@@ -60,7 +60,10 @@ WORKLOAD = {"C2": "batched 2D obstacle avoidance (test_obstacle_trajectory_2D sh
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline solve and of its evaluation and sampling records; the secondary "
+                         "records time fewer so the run stays short: the other configurations and the end-to-end record "
+                         "min(steps, 2), the other Jacobian mode 2, C1 5 calls")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default=HEADLINE, help="headline workload: C4 (default) | C2 | C3 | C5a | C5c")
@@ -72,7 +75,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline only: no sub-records for the other BASELINE configurations")
     ap.add_argument("--fused", action="store_true", help="one persistent solve kernel instead of lock-step stage kernels")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline solve returned (x, f, status, nit, violation of "
+                         "rank 0's batch) as DIR/<name>.npy in float64; batches whose outputs exceed 64 MB are "
+                         "represented by a fixed, seeded sample of problems")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def config_dict(name, B, L=None, jacobian="fd"):
@@ -243,6 +253,24 @@ def hist(a):
     return {str(k): int(v) for k, v in zip(*np.unique(np.asarray(a), return_counts=True))}
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+DUMP_SEED = 20261020
+
+
+def dump_outputs(path, outputs):
+    """Writes the per-problem output tensors as path/<name>.npy in float64 (the int32 ones convert exactly), so that two
+    builds can be compared output for output.  When the rows together exceed DUMP_LIMIT_BYTES, every array keeps the same rows:
+    a sorted sample drawn with DUMP_SEED, identical from run to run."""
+    host = {k: v.cpu().numpy().astype(np.float64) for k, v in outputs.items()}
+    B = len(host["x"])
+    row_bytes = sum(8 * (a.size // B) for a in host.values())
+    rows = min(B, (DUMP_LIMIT_BYTES - 4096) // row_bytes)        # 4 KiB of room for the .npy headers
+    idx = np.arange(B) if rows == B else np.sort(np.random.default_rng(DUMP_SEED).choice(B, rows, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a[idx]))
+
+
 # --------------------------------------------------------------------------------------------------------------
 # reference arm
 # --------------------------------------------------------------------------------------------------------------
@@ -364,6 +392,9 @@ def bench_config(G, name, B, steps, warmup, full=True):
     launches0 = G.lib.tg_launch_count()
     ms_step = G.timed(solve_step, steps, warmup, prepare=lambda: x.copy_(x0))
     solve_launches = (G.lib.tg_launch_count() - launches0) * steps // (steps + warmup)
+    if full and args.dump_outputs and G.rank == 0:
+        dump_outputs(args.dump_outputs, {"x": x, "f": bufs.f, "status": bufs.status, "nit": bufs.nit,
+                                         "violation": bufs.violation})
     value = G.world * B / (ms_step * 1e-3)
     status = bufs.status.cpu().numpy(); nit = bufs.nit.cpu().numpy()
     x_gpu = x.cpu().numpy()

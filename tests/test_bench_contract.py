@@ -1,5 +1,6 @@
-"""bench.py's contract on the CPU side: the reference arm prints one JSON line with the agreed keys, and the
-product arm refuses to run without a CUDA device (no CPU fallback)."""
+"""bench.py's contract: the reference arm prints one JSON line with the agreed keys, --dump-outputs writes a bounded
+sample that is the same from run to run and (GPU) equals what the headline solve returns, and the product arm refuses
+to run without a CUDA device (no CPU fallback)."""
 import json
 import os
 import subprocess
@@ -41,6 +42,44 @@ def test_reference_arm_prints_one_json_line(oracle_built):
     e2e = line["e2e"]
     assert e2e["value"] == line["value"] and e2e["unit"] == line["unit"]
     assert e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0
+
+
+def test_dump_outputs_is_a_bounded_reproducible_sample(tmp_path):
+    import numpy as np
+    import torch
+    import bench
+    B, n = 262144, 34                                   # the headline batch: its outputs exceed the 64 MB cap
+    out = {"x": torch.arange(B * n, dtype=torch.float64).reshape(B, n), "f": torch.arange(B, dtype=torch.float64),
+           "status": torch.arange(B, dtype=torch.int32) % 10, "nit": torch.arange(B, dtype=torch.int32)}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), out)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["f.npy", "nit.npy", "status.npy", "x.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    arr = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    rows = arr["nit"].astype(np.int64)
+    assert all(a.dtype == np.float64 and len(a) == len(rows) for a in arr.values()) and 0 < len(rows) < B
+    assert np.all(np.diff(rows) > 0)
+    assert np.array_equal(arr["x"], out["x"].numpy()[rows]) and np.array_equal(arr["status"], rows % 10)
+    assert all(np.array_equal(arr[f[:-4]], np.load(tmp_path / "b" / f)) for f in files)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_what_the_headline_solve_returns(native_lib, tmp_path):
+    """bench.py --dump-outputs on a small headline batch: the files equal a direct batch.solve of the same seeded batch"""
+    import numpy as np
+    import torch
+    import bench
+    from trajectory_generator_b200 import batch as tgb
+    proc = _run(["--quick", "--no-cpu-baseline", "--batch", "512", "--steps", "2", "--warmup", "1",
+                 "--dump-outputs", str(tmp_path)], timeout=600)
+    assert proc.returncode == 0, proc.stderr[-2000:]
+    bt = bench.make_batch("C4", 512)
+    dev = torch.device("cuda:0")
+    out = tgb.solve(bt.spec, torch.from_numpy(bt.par).to(dev), torch.from_numpy(bt.x0).to(dev), jacobian="fd")
+    assert sorted(os.listdir(tmp_path)) == sorted(k + ".npy" for k in out)
+    for k, v in out.items():
+        assert np.array_equal(np.load(tmp_path / (k + ".npy")), v.cpu().numpy().astype(np.float64)), k
 
 
 def test_product_arm_needs_a_cuda_device(native_lib):
