@@ -65,6 +65,13 @@ int tg_linear_rows_batch(const int *spec, int B, const double *par, double *alin
 
 /* bytes of device scratch tg_solve_batch needs for this shape and batch size */
 size_t tg_solve_workspace_bytes(const int *spec, int B);
+/* launch plan of the lock-step solve for this shape and batch size on the current device: out[0..6] = {lanes per problem
+ * of the line-search stage, lanes per problem of the QP stage, state staged in shared memory by the QP stage, QP
+ * scratch in global memory, line-search / derivative scratch in global memory, workspace slots, KiB of the slots}.
+ * Scratch goes to global memory (one workspace slot per resident lane group) only for shapes whose scratch does not
+ * fit in shared memory, or under the A/B switches TG_QP_FAR=1 / TG_LS_FAR=1.  Returns the number of values, or the
+ * negated error code (see tg_last_error). */
+int tg_solve_plan_info(const int *spec, int B, int *out, int cap);
 
 /*
  * M2: the per-problem scipy.optimize.minimize(method='SLSQP', options={'disp': False})

@@ -20,6 +20,9 @@ for item in sys.argv[3:]:
         bt = syn.make(name, B)
         cache[name] = (bt, torch.from_numpy(bt.par).to(dev), torch.from_numpy(bt.x0).to(dev), tgb.SolveBuffers(bt.spec, B, dev))
     bt, par, x0, bufs = cache[name]
+    if bufs.ws.numel() < lib.tg_solve_workspace_bytes(bufs.sp, B):      # a switch that adds workspace slots (TG_QP_FAR=1)
+        bufs = tgb.SolveBuffers(bt.spec, B, dev)
+        cache[name] = (bt, par, x0, bufs)
     ts = []
     for r in range(reps + 1):
         x = x0.clone()

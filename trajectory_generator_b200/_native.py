@@ -94,6 +94,8 @@ def lib():
         L.tg_linear_rows_batch.argtypes = [_I32, ctypes.c_int, vp, vp, vp]
         L.tg_solve_workspace_bytes.argtypes = [_I32, ctypes.c_int]
         L.tg_solve_workspace_bytes.restype = sz
+        L.tg_solve_plan_info.argtypes = [_I32, ctypes.c_int, _I32, ctypes.c_int]
+        L.tg_solve_plan_info.restype = ctypes.c_int
         L.tg_solve_batch.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_double,
                                      ctypes.c_int, vp, sz, vp]
         L.tg_eval_host.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp, vp]

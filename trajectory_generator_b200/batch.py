@@ -88,6 +88,21 @@ class SolveBuffers:
         self.ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
+PLAN_FIELDS = ("gs_ls", "gs_qp", "staged", "qp_far", "ls_far", "slots", "slot_kib")
+
+
+def solve_plan(spec, B):
+    """Launch plan of the lock-step solve of B problems of this shape on the current device (tg_solve_plan_info): lanes
+    per problem of the line-search and QP stages, whether the QP stage stages the state in shared memory, whether the
+    QP / line-search scratch lives in workspace slots (shapes whose scratch does not fit in shared memory), the number
+    of slots and their KiB.  A dict keyed by PLAN_FIELDS."""
+    spec, sp = _native.spec_ptr(spec)
+    out = np.zeros(len(PLAN_FIELDS), dtype=np.int32)
+    cnt = _native.lib().tg_solve_plan_info(sp, int(B), out.ctypes.data_as(_native._I32), out.size)
+    _native.check(-cnt if cnt < 0 else 0, "tg_solve_plan_info")
+    return {k: int(v) for k, v in zip(PLAN_FIELDS, out)}
+
+
 def _flags(jacobian, fused):
     return JACOBIAN_MODES[jacobian] | (2 if fused else 0)
 

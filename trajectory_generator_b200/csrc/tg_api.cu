@@ -163,6 +163,11 @@ struct TgSolvePlan {
     size_t np, smem_ls, smem_qp;
     int staged, chunk, gs_ls, gs_qp;
     size_t phased_bytes;
+    // scratch of the QP / line-search and derivative stages in workspace slots instead of shared memory; the stages
+    // run one after the other on one stream, so they share the slots: `slots` of the stage with more lane groups,
+    // `slot_bytes` of the larger need (multiple of 256)
+    int qp_far, ls_far, slots;
+    size_t slot_bytes;
 };
 
 #define TG_PHASED_CHUNK_BYTES ((size_t)6 << 30)     // cap of the global state per chunk (the batch is solved in chunks)
@@ -209,7 +214,11 @@ static int tg_plan_solve(const TgShape &S, int B, TgSolvePlan *P)
         if (P->smem_ls * 2 <= sm_total - 2048 || gs == 32) break;
         gs *= 2;
     }
-    if (P->smem_ls > budget) return tg_fail(3, "problem shape too large for the line-search kernel's shared memory");
+    // shapes whose share does not fit (TG_LS_FAR=1: any shape, for A/B runs): parameters and state prefix read in place,
+    // evaluation scratch in workspace slots, 32 lanes per problem
+    const char *lsf = getenv("TG_LS_FAR");
+    P->ls_far = P->smem_ls > budget || (lsf && atoi(lsf) != 0);
+    if (P->ls_far) { gs = 32; P->smem_ls = 0; }
     P->gs_ls = gs;
     // QP: lanes per problem from the variables of the subproblem after the elimination of the terminal location rows
     // (tg_sqp_qp_dim): 16, one warp, or two warps (64 lanes) beyond 32, so that every lane-strided loop takes one pass.  Persistent state staged through shared memory when 16 problems still fit.
@@ -221,19 +230,35 @@ static int tg_plan_solve(const TgShape &S, int B, TgSolvePlan *P)
         gs = v ? atoi(v) : (tg_sqp_qp_dim(S.L) > 32 ? 64 : (tg_sqp_qp_dim(S.L) > 16 || nd > 4) ? 32 : 16);
         if (!(gs == 8 || gs == 16 || gs == 32 || gs == 64)) gs = 32;
     }
-    P->gs_qp = gs;
     const size_t with_state = gs == 64 ? tg_qp_smem_g64(S, 1) : TG_DISPATCH(gs, tg_qp_smem_g8(S, 1), tg_qp_smem_g16(S, 1), tg_qp_smem_g32(S, 1));
     const size_t without = gs == 64 ? tg_qp_smem_g64(S, 0) : TG_DISPATCH(gs, tg_qp_smem_g8(S, 0), tg_qp_smem_g16(S, 0), tg_qp_smem_g32(S, 0));
     // (16-lane groups: 8 problems per CTA, never staged by this rule -- measured: C5 239 ms unstaged, 260 ms staged)
     P->staged = with_state * 4 <= sm_total - 4096;
     if (const char *v = getenv("TG_QP_STAGED")) P->staged = atoi(v) != 0 && with_state <= budget;      // tuning override
     P->smem_qp = P->staged ? with_state : without;
-    if (P->smem_qp > budget) return tg_fail(3, "problem shape too large for the QP kernel's shared memory");
+    // shapes whose scratch does not fit even unstaged (TG_QP_FAR=1: any shape, for A/B runs): scratch in workspace
+    // slots, state in global memory, 64 lanes per problem
+    const char *qpf = getenv("TG_QP_FAR");
+    P->qp_far = P->smem_qp > budget || (qpf && atoi(qpf) != 0);
+    if (P->qp_far) { gs = 64; P->staged = 0; P->smem_qp = 0; }
+    P->gs_qp = gs;
+    // (a state of tens of MB per problem -- 3-D, N = 512 -- makes chunks of fewer than 1024 problems: the cap holds)
     size_t chunk = TG_PHASED_CHUNK_BYTES / (P->np * sizeof(double));
-    if (chunk < 1024) chunk = 1024;
+    if (chunk < 1) chunk = 1;
     if (chunk > (size_t)B) chunk = (size_t)B;
     P->chunk = (int)chunk;
     P->phased_bytes = chunk * P->np * sizeof(double);
+    // workspace slots: one per lane group of a grid capped at TG_FAR_CTAS_PER_SM CTAs per SM and at the chunk's work
+    // (far-placed shapes run as one slice: tg_solve_phased)
+    auto slots_of = [&](int groups) {
+        const size_t need = (chunk + groups - 1) / groups, cap = (size_t)g_sm_count * TG_FAR_CTAS_PER_SM;
+        return (need < cap ? need : cap) * groups;
+    };
+    const size_t qp_slots = P->qp_far ? slots_of(128 / 64) : 0, ls_slots = P->ls_far ? slots_of(128 / 32) : 0;
+    const size_t qp_bytes = qp_slots * tg_sqp_qp_scratch_doubles(S.L) * sizeof(double);
+    const size_t ls_bytes = ls_slots * tg_sqp_ls_slot_doubles(S.L) * sizeof(double);
+    P->slots = (int)(qp_slots > ls_slots ? qp_slots : ls_slots);
+    P->slot_bytes = ((qp_bytes > ls_bytes ? qp_bytes : ls_bytes) + 255) & ~(size_t)255;
     return 0;
 }
 
@@ -243,8 +268,20 @@ extern "C" size_t tg_solve_workspace_bytes(const int *spec, int B)
     TgShape S;
     TgSolvePlan P;
     if (tg_make_shape(spec, &S) || tg_plan_solve(S, B, &P)) return 0;
-    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk);
+    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk) + P.slot_bytes;
     return (P.global_bytes > phased ? P.global_bytes : phased) + 4 * TG_ROUNDCTL_BYTES;
+}
+
+extern "C" int tg_solve_plan_info(const int *spec, int B, int *out, int cap)
+{
+    TgShape S;
+    TgSolvePlan P;
+    int rc = tg_make_shape(spec, &S);
+    if (!rc) rc = tg_plan_solve(S, B > 0 ? B : 1, &P);
+    if (rc) return -rc;
+    const int v[7] = {P.gs_ls, P.gs_qp, P.staged, P.qp_far, P.ls_far, P.slots, (int)(P.slot_bytes >> 10)};
+    for (int i = 0; i < 7 && out && i < cap; i++) out[i] = v[i];
+    return 7;
 }
 
 #define TG_LAUNCH(call, what)                                                   \
@@ -276,7 +313,8 @@ extern "C" int tg_last_solve_stats(double *out, int cap)
     return 6;
 }
 
-// device bookkeeping in front of the per-problem state: [TgRoundCtl x TG_MAX_SLICES | list0[chunk] | list1[chunk]]
+// device bookkeeping in front of the per-problem state: [TgRoundCtl x TG_MAX_SLICES | list0[chunk] | list1[chunk] |
+// workspace slots (far-placed stages only)]
 #define TG_MAX_SLICES 4
 #define TG_HEADER_BYTES (TG_MAX_SLICES * TG_ROUNDCTL_BYTES)
 static size_t tg_lists_bytes(int chunk) { return (((size_t)2 * chunk * sizeof(int)) + 255) & ~(size_t)255; }
@@ -335,7 +373,9 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
     const TgLayout &L = S.L;
     char *wsb = (char *)workspace;
     int *list_base = (int *)(wsb + TG_HEADER_BYTES);
-    double *pws_base = (double *)(wsb + TG_HEADER_BYTES + tg_lists_bytes(P.chunk));
+    double *far = (double *)(wsb + TG_HEADER_BYTES + tg_lists_bytes(P.chunk));
+    double *pws_base = (double *)((char *)far + P.slot_bytes);
+    double *far_qp = P.qp_far ? far : nullptr, *far_ls = P.ls_far ? far : nullptr;
     const bool timing = g_stage_timing.load() != 0;
     std::vector<cudaEvent_t> ev;
     if (timing) g_stats = TgSolveStats{0, 0, 0, 0, 0, 0};
@@ -351,6 +391,7 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
     // problems), -2 % on C3, +3 % on C5a, +8 % on C4 (state in L2 / HBM): two when the state is staged in shared memory
     int want = P.staged ? 2 : 1;
     if (const char *v = getenv("TG_SLICES")) want = atoi(v);
+    if (P.slot_bytes) want = 1;          // the workspace slots serve one grid at a time
     if (want < 1) want = 1;
     if (want > TG_MAX_SLICES) want = TG_MAX_SLICES;
     TgSliceLease lease;
@@ -389,19 +430,19 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
                 any = true;
                 const double *cpar = par + (size_t)(lo + q.lo) * L.P;
                 TG_CUDA(mark());
-                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_ls_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                      tg_launch_ls_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                      tg_launch_ls_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
+                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_ls_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
+                                      tg_launch_ls_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
+                                      tg_launch_ls_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
                           "tg_sqp_ls_kernel");
-                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_fd_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                          tg_launch_fd_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                          tg_launch_fd_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
+                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_fd_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
+                                          tg_launch_fd_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
+                                          tg_launch_fd_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
                           "tg_sqp_der_kernel");
                 TG_CUDA(mark());
-                TG_LAUNCH(P.gs_qp == 64 ? tg_launch_qp_g64(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st) :
-                          TG_DISPATCH(P.gs_qp, tg_launch_qp_g8(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
-                                      tg_launch_qp_g16(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
-                                      tg_launch_qp_g32(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st)),
+                TG_LAUNCH(P.gs_qp == 64 ? tg_launch_qp_g64(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st) :
+                          TG_DISPATCH(P.gs_qp, tg_launch_qp_g8(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
+                                      tg_launch_qp_g16(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
+                                      tg_launch_qp_g32(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st)),
                           "tg_sqp_qp_kernel");
                 TG_CUDA(mark());
             }
@@ -456,9 +497,7 @@ extern "C" int tg_solve_batch(const int *spec, int B, const double *par, double 
     if (rc) return rc;
     if (B <= 0) return 0;
     if ((rc = tg_plan_solve(S, B, &P))) return rc;
-    // (shapes with more than 63 variables run the 64-lane QP kernel with two passes per lane-strided loop; the limit is the
-    // shared memory of the QP stage, checked by tg_plan_solve)
-    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk);
+    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk) + P.slot_bytes;
     const size_t need = (P.global_bytes > phased ? P.global_bytes : phased) + TG_HEADER_BYTES;
     if (!workspace || workspace_bytes < need) return tg_fail(4, "workspace too small (see tg_solve_workspace_bytes)");
     int *counters = (int *)workspace;

@@ -72,6 +72,14 @@ struct TgRoundCtl {
 };
 #define TG_ROUNDCTL_BYTES 256
 
+// Shapes whose per-problem scratch does not fit in shared memory run stage kernels that take it from the solve
+// workspace instead: one slot per resident lane group (the grids are persistent, a group reuses its slot for every
+// problem it pulls).  Their grids are capped at TG_FAR_CTAS_PER_SM CTAs per SM, so that the slot count is known before
+// the launch (tg_plan_solve sizes the workspace); that is also their launch bound, which leaves them 256 registers a
+// thread (no spills) and keeps the slots of a large shape few.  Only the generic instantiations exist: the QP kernel with 64 lanes
+// (tg_solve_g64.cu), the line-search and derivative kernels with 32 (tg_solve_g32.cu, tg_solve_fd_g32.cu).
+#define TG_FAR_CTAS_PER_SM 2
+
 // Every kernel with dynamic shared memory is allowed the device's opt-in maximum (not the size of the launch at
 // hand: launches of one kernel with different sizes may be issued from several host threads, tg_solve_mixed_host).
 // Done once per (device, kernel).
@@ -107,8 +115,9 @@ static inline cudaError_t tg_allow_shared_memory(K kernel)
     cudaError_t tg_launch_begin##SFX(const TgShape &S, int B, const double *x, double *pws, size_t np, int maxiter,       \
                                      double ftol, int flags, TgRoundCtl *rc, int *list0, cudaStream_t st);                \
     cudaError_t tg_launch_ls##SFX(const TgShape &S, int B, const double *par, double *pws, size_t np, size_t smem,        \
-                                  TgRoundCtl *rc, const int *list, int parity, int sm_count, cudaStream_t st);            \
-    cudaError_t tg_launch_qp##SFX(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem,               \
+                                  double *far, TgRoundCtl *rc, const int *list, int parity, int sm_count,                 \
+                                  cudaStream_t st);                                                                       \
+    cudaError_t tg_launch_qp##SFX(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem, double *far,  \
                                   TgRoundCtl *rc, const int *list, int *next, int parity, int sm_count, cudaStream_t st); \
     size_t tg_ls_smem##SFX(const TgShape &S);                                                                             \
     size_t tg_qp_smem##SFX(const TgShape &S, int staged);                                                                 \
@@ -122,14 +131,14 @@ TG_DECLARE_VARIANT(_g32)
 // finite-difference stage (tg_solve_fd_g*.cu): value-only evaluators inlined, one kernel of its own
 #define TG_DECLARE_FD(SFX)                                                                                              \
     cudaError_t tg_launch_fd##SFX(const TgShape &S, int B, const double *par, double *pws, size_t np, size_t smem,      \
-                                  TgRoundCtl *rc, const int *list, int parity, int sm_count, cudaStream_t st);
+                                  double *far, TgRoundCtl *rc, const int *list, int parity, int sm_count, cudaStream_t st);
 TG_DECLARE_FD(_g8)
 TG_DECLARE_FD(_g16)
 TG_DECLARE_FD(_g32)
 
 // QP stage with 64 lanes per problem (tg_solve_g64.cu)
-cudaError_t tg_launch_qp_g64(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem, TgRoundCtl *rc,
-                             const int *list, int *next, int parity, int sm_count, cudaStream_t st);
+cudaError_t tg_launch_qp_g64(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem, double *far,
+                             TgRoundCtl *rc, const int *list, int *next, int parity, int sm_count, cudaStream_t st);
 size_t tg_qp_smem_g64(const TgShape &S, int staged);
 
 // launch counter of the library (tg_launch_count), for kernels launched outside tg_api.cu

@@ -239,6 +239,9 @@ TG_HD void tg_sqp_carve2(const TgLayout &L, double *pbase, double *sbase, TgSqpW
 
 // scratch needed by the line-search stage alone (cf + the evaluators' scratch) / by the QP stage alone
 TG_HD size_t tg_sqp_ls_scratch_doubles(const TgLayout &L) { return (size_t)L.r_turn + 1 + tg_scratch_doubles(L); }
+// workspace slot of one lane group of the line-search / derivative kernels with their scratch in global memory: the
+// evaluation scratch, padded to an even count (slots stay 16-byte aligned)
+TG_HD size_t tg_sqp_ls_slot_doubles(const TgLayout &L) { const size_t e = tg_sqp_ls_scratch_doubles(L); return e + (e & 1); }
 // front of the persistent block that the derivative stage touches: [ctl | x xl xu g | c], even
 TG_HD size_t tg_sqp_prefix_fd_doubles(const TgLayout &L)
 {
