@@ -626,31 +626,36 @@ class OracleProblem:
     def grad_fd(self, x):
         return self.jac_fd(x, fun=lambda z: np.atleast_1d(self.fun(z)))[0]
 
-    def jac_central(self, x, fun=None, h=1e-4, order=4):
+    def jac_central(self, x, fun=None, h=1e-4, order=4, cols=None):
         """Jacobian oracle: central differences of the oracle closures, 4th order (5-point stencil) or 6th order
-        (7-point stencil).  Only meaningful where the active branches are stable over the whole stencil."""
+        (7-point stencil).  Only meaningful where the active branches are stable over the whole stencil.
+        cols: the columns to difference (default all); the result has one column per entry of cols."""
         fun = self.cons if fun is None else fun
         x = np.asarray(x, dtype=float)
+        cols = np.arange(self.n) if cols is None else np.asarray(cols, dtype=int)
         m = len(np.atleast_1d(fun(x)))
-        J = np.zeros((m, self.n))
+        J = np.zeros((m, len(cols)))
         weights = {4: ((1, 8.0 / 12), (2, -1.0 / 12)), 6: ((1, 45.0 / 60), (2, -9.0 / 60), (3, 1.0 / 60))}[order]
-        for i in range(self.n):
+        for col, i in enumerate(cols):
             hh = h * max(1.0, abs(x[i]))
             e = np.zeros(self.n); e[i] = hh
             with np.errstate(all="ignore"):
                 acc = 0.0
                 for k, w in weights:
                     acc = acc + w * (np.atleast_1d(fun(x + k * e)) - np.atleast_1d(fun(x - k * e)))
-                J[:, i] = acc / hh
+                J[:, col] = acc / hh
         return J
 
-    def jacobian_error(self, J, x, fun=None):
+    def jacobian_error(self, J, x, fun=None, cols=None):
         """Element-wise relative error of J against the Jacobian oracle, and the mask of entries the oracle can
         vouch for.  Two independent 6th-order estimates (h = 1e-3 and 2.5e-4) must agree with each other to 1e-10
         for an entry to be trusted: where they do not, a stencil straddles a kink of the reference's piecewise
         smooth closures (max/min over intervals, hull points, root in/out of the interval; SURVEY.md 8(c)) and no
-        finite-difference oracle exists for that entry."""
-        est = [self.jac_central(x, fun=fun, h=h, order=6) for h in (1e-3, 2.5e-4)]
+        finite-difference oracle exists for that entry.  cols: check only these columns of J (default all); the
+        results then have one column per entry of cols."""
+        if cols is not None:
+            J = np.asarray(J)[..., cols]
+        est = [self.jac_central(x, fun=fun, h=h, order=6, cols=cols) for h in (1e-3, 2.5e-4)]
         with np.errstate(all="ignore"):
             scale = np.maximum(1.0, np.abs(est[1]))
             trusted = np.abs(est[0] - est[1]) <= 1e-10 * scale

@@ -130,6 +130,13 @@ extern "C" int tg_eval_batch(const int *spec, int B, const double *par, const do
     if (B <= 0) return 0;
     if ((rc = tg_device_check())) return rc;
     const int gs = tg_env_gs("TG_EVAL_GS", tg_default_gs(S.L));
+    // (a CTA runs fewer lane groups where 128 / gs do not fit; one must)
+    const size_t need = (size_t)tg_eval_group_doubles(S.L, c == nullptr) * sizeof(double);
+    if (need > (size_t)g_smem_optin) {
+        snprintf(g_err, sizeof g_err, "tg_eval_kernel: a problem with n = %d, m = %d needs %zu bytes of shared memory, "
+                 "more than the device's %d", S.L.n, S.L.m, need, g_smem_optin);
+        return 3;
+    }
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = TG_DISPATCH(gs, tg_launch_eval_g8(S, B, par, x, f, g, c, jnl, g_sm_count, g_smem_optin, st),
                                 tg_launch_eval_g16(S, B, par, x, f, g, c, jnl, g_sm_count, g_smem_optin, st),

@@ -1217,6 +1217,15 @@ TG_FN void tg_rows_obstacles(const TgLayout &L, const int *sp, const double *par
 // sweeps (tg_fd_turning / tg_fd_obstacles) 4 perturbed values per control-point variable + 2 per interval
 TG_HD int tg_scratch_doubles(const TgLayout &L) { return (L.n_obs * L.nint > 0 ? L.n_obs * L.nint : 1) + 4 * L.d * L.N + 2 * L.nint + 2; }
 
+// shared memory of one problem in the evaluation kernel (tg_kernels_eval.inc): variables, parameters, the evaluators'
+// scratch and -- only when the caller does not ask for the constraint values -- a sink for them.  (The evaluators only
+// WRITE constraint rows, so with `c` given they write straight to global memory: the corridor rows, most of C4's 209,
+// leave the lanes as contiguous runs.)
+TG_HD int tg_eval_group_doubles(const TgLayout &L, bool sink_c)
+{
+    return L.n + L.P + (sink_c ? L.m : 0) + tg_scratch_doubles(L) + 4;
+}
+
 // zero every nonlinear Jacobian row (they are rewritten sparsely on each evaluation)
 TG_FN void tg_zero_nonlinear_rows(const TgLayout &L, const TgJac &J)
 {

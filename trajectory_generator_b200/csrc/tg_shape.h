@@ -15,7 +15,9 @@ struct TgShape {
 // kernel argument (any shape); k > 0 = the descriptor is the compile-time constant below, so the whole TgLayout
 // (sizes, row / parameter offsets, which constraint blocks exist) folds into the code: workspace arrays sit at
 // constant offsets, absent constraint kinds are compiled out, loop bounds are known.  Same arithmetic in the same
-// order: results are bit-identical to the generic instantiation.  The list holds the BASELINE.json configurations
+// order, but the compiler contracts the folded code into FMAs differently in places: the objective and its gradient
+// are bit-identical to the generic instantiation, constraint rows and their Jacobian may differ in the last places
+// (C4: bit-identical throughout; tests/test_eval_sweep.py).  The list holds the BASELINE.json configurations
 // (trajectory_generator_b200/synthetic.py builds the same descriptors; tests/test_packing.py compares them).
 // ---------------------------------------------------------------------------
 #define TG_FIXED_SHAPES 5
@@ -111,7 +113,7 @@ static inline cudaError_t tg_allow_shared_memory(K kernel)
                                     double *c, double *jnl, int sm_count, int smem_optin, cudaStream_t st);               \
     cudaError_t tg_launch_linear##SFX(const TgShape &S, int B, const double *par, double *alin, int sm_count,             \
                                       cudaStream_t st);                                                                   \
-    size_t tg_eval_smem##SFX(const TgShape &S, bool sink_c);                                                                           \
+    size_t tg_eval_smem##SFX(const TgShape &S, bool sink_c, int smem_optin);                                              \
     cudaError_t tg_launch_begin##SFX(const TgShape &S, int B, const double *x, double *pws, size_t np, int maxiter,       \
                                      double ftol, int flags, TgRoundCtl *rc, int *list0, cudaStream_t st);                \
     cudaError_t tg_launch_ls##SFX(const TgShape &S, int B, const double *par, double *pws, size_t np, size_t smem,        \
