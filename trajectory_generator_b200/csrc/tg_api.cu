@@ -1,12 +1,17 @@
 // Host side of the C-ABI declared in include/trajectory_generator_b200.h, plus the single-problem kernels
 // behind the reference's 24 legacy symbols.
 //
-// Device code lives in per-group-size translation units (a problem is worked on by 8, 16 or 32 lanes):
-//   tg_eval_g*.cu   M1: objective, gradient, constraint rows, analytic nonlinear Jacobian rows
-//   tg_solve_g*.cu  M2: the SLSQP iteration (tg_sqp.h) as lock-step stage kernels (+ the fused kernel, g32)
+// Device code lives in per-group-size translation units (a problem is worked on by 8, 16, 32 or 64 lanes):
+//   tg_eval_g*.cu      M1: objective, gradient, constraint rows, analytic nonlinear Jacobian rows
+//   tg_solve_g*.cu     M2: the SLSQP iteration (tg_sqp.h) as lock-step stage kernels: line search, QP stage
+//   tg_solve_fd_g*.cu  M2: the derivative stage
+//   tg_solve_fused.cu  M2 as one kernel (kept for comparison)
+// The plans here (tg_plan_solve, tg_eval_batch) make every launch decision -- lanes, shared memory, placement,
+// staging, slices, fixed-shape instantiation -- and read the tuning overrides; the units' launchers execute them.
 // Data layout in HBM: row-major [B][n] variables, [B][P] parameters, [B][m] rows, [B][m_nl][n] Jacobians --
 // a lane group reads/writes its problem's rows as contiguous 8-byte accesses; per-problem working sets are
 // staged in shared memory.
+#include <assert.h>
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -104,7 +109,7 @@ void tg_note_launch(int count) { g_launches += (unsigned long long)count; }
 
 // ---------------------------------------------------------------------------
 // lanes per problem.  Heuristic: enough lanes for the per-interval terms (the longest per-lane chains), capped by
-// what shared memory allows; TG_EVAL_GS / TG_LS_GS / TG_QP_GS (8, 16, 32) override for tuning.
+// what shared memory allows; TG_EVAL_GS / TG_LS_GS (8, 16, 32) and TG_QP_GS (16, 32, 64) override for tuning.
 // ---------------------------------------------------------------------------
 static int tg_env_gs(const char *name, int dflt)
 {
@@ -119,7 +124,16 @@ static int tg_default_gs(const TgLayout &L)
     return L.nint <= 8 ? 8 : (L.nint <= 16 ? 16 : 32);
 }
 
-#define TG_DISPATCH(gs, call8, call16, call32) ((gs) == 8 ? (call8) : (gs) == 16 ? (call16) : (call32))
+// launchers of a kernel family by lanes per problem (8, 16, 32, 64); nullptr: no such kernel, never planned
+static int tg_lanes_index(int lanes) { return lanes == 8 ? 0 : lanes == 16 ? 1 : lanes == 32 ? 2 : 3; }
+typedef cudaError_t (*TgStageLauncher)(const TgStageLaunch &);
+static const TgStageLauncher tg_ls_launchers[4] = {tg_launch_ls_g8, tg_launch_ls_g16, tg_launch_ls_g32, nullptr};
+static const TgStageLauncher tg_fd_launchers[4] = {tg_launch_fd_g8, tg_launch_fd_g16, tg_launch_fd_g32, nullptr};
+static const TgStageLauncher tg_qp_launchers[4] = {nullptr, tg_launch_qp_g16, tg_launch_qp_g32, tg_launch_qp_g64};
+static cudaError_t (*const tg_eval_launchers[3])(const TgEvalLaunch &) = {tg_launch_eval_g8, tg_launch_eval_g16, tg_launch_eval_g32};
+
+// fixed-shape instantiation of a shape (tg_shape.h); TG_GENERIC_KERNELS: the generic ones, for A/B runs
+static int tg_plan_fix(const TgShape &S) { return getenv("TG_GENERIC_KERNELS") ? 0 : tg_fixed_index(S.sp); }
 
 extern "C" int tg_eval_batch(const int *spec, int B, const double *par, const double *x, double *f, double *g,
                              double *c, double *jnl, void *stream)
@@ -131,16 +145,17 @@ extern "C" int tg_eval_batch(const int *spec, int B, const double *par, const do
     if ((rc = tg_device_check())) return rc;
     const int gs = tg_env_gs("TG_EVAL_GS", tg_default_gs(S.L));
     // (a CTA runs fewer lane groups where 128 / gs do not fit; one must)
+    const int groups = tg_eval_groups(S.L, gs, c == nullptr, g_smem_optin);
     const size_t need = (size_t)tg_eval_group_doubles(S.L, c == nullptr) * sizeof(double);
-    if (need > (size_t)g_smem_optin) {
+    if (groups == 0) {
         snprintf(g_err, sizeof g_err, "tg_eval_kernel: a problem with n = %d, m = %d needs %zu bytes of shared memory, "
                  "more than the device's %d", S.L.n, S.L.m, need, g_smem_optin);
         return 3;
     }
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = TG_DISPATCH(gs, tg_launch_eval_g8(S, B, par, x, f, g, c, jnl, g_sm_count, g_smem_optin, st),
-                                tg_launch_eval_g16(S, B, par, x, f, g, c, jnl, g_sm_count, g_smem_optin, st),
-                                tg_launch_eval_g32(S, B, par, x, f, g, c, jnl, g_sm_count, g_smem_optin, st));
+    int grid = (B + groups - 1) / groups;
+    if (grid > g_sm_count * 32) grid = g_sm_count * 32;
+    const TgEvalLaunch a = {S, B, par, x, f, g, c, jnl, tg_plan_fix(S), grid, groups, groups * need, (cudaStream_t)stream};
+    cudaError_t e = tg_eval_launchers[tg_lanes_index(gs)](a);
     g_launches++;
     if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_eval_kernel launch", e);
     return 0;
@@ -160,20 +175,25 @@ extern "C" int tg_linear_rows_batch(const int *spec, int B, const double *par, d
 }
 
 // ---------------------------------------------------------------------------
-// M2 launch plans
+// M2 launch plan of the lock-step solve: every launch decision of tg_solve_phased, and the workspace it carves
 // ---------------------------------------------------------------------------
+#define TG_MAX_SLICES 4
+struct TgStagePlan {
+    int lanes, far;         // far: scratch in workspace slots instead of shared memory
+    size_t smem;            // dynamic shared memory per CTA
+};
 struct TgSolvePlan {
-    // fused kernel
-    int warps_per_cta, ctas, use_global;
-    size_t ws_doubles, smem_bytes, global_bytes;
-    // lock-step kernels
-    size_t np, smem_ls, smem_qp;
-    int staged, chunk, gs_ls, gs_qp;
+    int fix;                // fixed-shape instantiation (tg_shape.h), 0 = generic
+    TgStagePlan ls, der, qp;
+    int staged;             // QP stage: persistent state staged through shared memory
+    int slices;             // independent slices of a chunk of at least 8,192 problems (tg_solve_phased)
+    size_t np;              // doubles of persistent state per problem
+    int chunk;              // problems per chunk (the batch is solved in chunks)
     size_t phased_bytes;
     // scratch of the QP / line-search and derivative stages in workspace slots instead of shared memory; the stages
     // run one after the other on one stream, so they share the slots: `slots` of the stage with more lane groups,
     // `slot_bytes` of the larger need (multiple of 256)
-    int qp_far, ls_far, slots;
+    int slots;
     size_t slot_bytes;
 };
 
@@ -183,72 +203,44 @@ static int tg_plan_solve(const TgShape &S, int B, TgSolvePlan *P)
 {
     int rc = tg_device_check();
     if (rc) return rc;
+    const TgLayout &L = S.L;
     const size_t budget = (size_t)g_smem_optin - 1024;
     const size_t sm_total = 227 * 1024;
-    // ---- fused: shared-memory workspace when at least 8 warps fit on an SM, else global workspace
-    P->ws_doubles = tg_sqp_workspace_doubles(S.L);
-    const size_t per_warp_shared = (S.L.P + P->ws_doubles + 2) * sizeof(double);
-    if (per_warp_shared * 8 <= sm_total) {
-        P->use_global = 0;
-        P->warps_per_cta = 4;
-        while (per_warp_shared * P->warps_per_cta > budget) P->warps_per_cta >>= 1;
-        P->smem_bytes = per_warp_shared * P->warps_per_cta;
-        int per_sm = (int)(sm_total / (P->smem_bytes + 1024));
-        if (per_sm < 1) per_sm = 1;
-        if (per_sm * P->warps_per_cta > 32) per_sm = 32 / P->warps_per_cta;
-        P->ctas = g_sm_count * per_sm;
-        P->global_bytes = 0;
-    } else {
-        P->use_global = 1;
-        P->warps_per_cta = 4;
-        P->smem_bytes = (size_t)P->warps_per_cta * (S.L.P + 2) * sizeof(double);
-        P->ctas = g_sm_count * 4;
-        P->global_bytes = (size_t)P->ctas * P->warps_per_cta * P->ws_doubles * sizeof(double);
-    }
-    const int need = (B + P->warps_per_cta - 1) / P->warps_per_cta;
-    if (P->ctas > need) {
-        P->ctas = need > 0 ? need : 1;
-        if (P->use_global) P->global_bytes = (size_t)P->ctas * P->warps_per_cta * P->ws_doubles * sizeof(double);
-    }
-    // ---- lock step
-    P->np = tg_sqp_persistent_doubles(S.L);
+    P->fix = tg_plan_fix(S);
+    P->np = tg_sqp_persistent_doubles(L);
     // line search: smallest group that leaves >= 8 resident warps' worth of shared memory per SM
     // (shapes with more than 32 variables: 16 lanes at least -- C4 fits 8-lane groups since its derivative stage stages
     // less, but runs 3 % slower with them)
-    int gs = tg_env_gs("TG_LS_GS", S.L.n > 32 && tg_default_gs(S.L) < 16 ? 16 : tg_default_gs(S.L));
-    for (;;) {
-        P->smem_ls = TG_DISPATCH(gs, tg_ls_smem_g8(S), tg_ls_smem_g16(S), tg_ls_smem_g32(S));
-        if (P->smem_ls * 2 <= sm_total - 2048 || gs == 32) break;
-        gs *= 2;
-    }
+    int gs = tg_env_gs("TG_LS_GS", L.n > 32 && tg_default_gs(L) < 16 ? 16 : tg_default_gs(L));
+    while (tg_ls_smem_bytes(L, gs) * 2 > sm_total - 2048 && gs < 32) gs *= 2;
     // shapes whose share does not fit (TG_LS_FAR=1: any shape, for A/B runs): parameters and state prefix read in place,
     // evaluation scratch in workspace slots, 32 lanes per problem
     const char *lsf = getenv("TG_LS_FAR");
-    P->ls_far = P->smem_ls > budget || (lsf && atoi(lsf) != 0);
-    if (P->ls_far) { gs = 32; P->smem_ls = 0; }
-    P->gs_ls = gs;
+    const int ls_far = tg_ls_smem_bytes(L, gs) > budget || (lsf && atoi(lsf) != 0);
+    if (ls_far) gs = 32;
+    // (the derivative stage stages less than the line search: shared memory of its own)
+    P->ls = {gs, ls_far, ls_far ? 0 : tg_ls_smem_bytes(L, gs)};
+    P->der = {gs, ls_far, ls_far ? 0 : tg_fd_smem_bytes(L, gs)};
     // QP: lanes per problem from the variables of the subproblem after the elimination of the terminal location rows
     // (tg_sqp_qp_dim): 16, one warp, or two warps (64 lanes) beyond 32, so that every lane-strided loop takes one pass.  Persistent state staged through shared memory when 16 problems still fit.
     {
         const char *v = getenv("TG_QP_GS");
         // (16 lanes run with the state in global memory: only shapes with few dense inequality rows, whose copy sits next
         // to the scratch -- C5: 239 ms against 276 ms with 32 lanes; C2, 11 such rows: 184 ms against 176 ms)
-        const int nd = S.L.m - 2 * S.L.n_sfc - S.L.meq;
-        gs = v ? atoi(v) : (tg_sqp_qp_dim(S.L) > 32 ? 64 : (tg_sqp_qp_dim(S.L) > 16 || nd > 4) ? 32 : 16);
-        if (!(gs == 8 || gs == 16 || gs == 32 || gs == 64)) gs = 32;
+        const int nd = L.m - 2 * L.n_sfc - L.meq;
+        gs = v ? atoi(v) : (tg_sqp_qp_dim(L) > 32 ? 64 : (tg_sqp_qp_dim(L) > 16 || nd > 4) ? 32 : 16);
+        if (!(gs == 16 || gs == 32 || gs == 64)) gs = 32;        // TG_QP_GS: 16, 32 or 64 (the QP kernels there are); else 32
     }
-    const size_t with_state = gs == 64 ? tg_qp_smem_g64(S, 1) : TG_DISPATCH(gs, tg_qp_smem_g8(S, 1), tg_qp_smem_g16(S, 1), tg_qp_smem_g32(S, 1));
-    const size_t without = gs == 64 ? tg_qp_smem_g64(S, 0) : TG_DISPATCH(gs, tg_qp_smem_g8(S, 0), tg_qp_smem_g16(S, 0), tg_qp_smem_g32(S, 0));
+    const size_t with_state = tg_qp_smem_bytes(L, gs, 1), without = tg_qp_smem_bytes(L, gs, 0);
     // (16-lane groups: 8 problems per CTA, never staged by this rule -- measured: C5 239 ms unstaged, 260 ms staged)
     P->staged = with_state * 4 <= sm_total - 4096;
     if (const char *v = getenv("TG_QP_STAGED")) P->staged = atoi(v) != 0 && with_state <= budget;      // tuning override
-    P->smem_qp = P->staged ? with_state : without;
     // shapes whose scratch does not fit even unstaged (TG_QP_FAR=1: any shape, for A/B runs): scratch in workspace
     // slots, state in global memory, 64 lanes per problem
     const char *qpf = getenv("TG_QP_FAR");
-    P->qp_far = P->smem_qp > budget || (qpf && atoi(qpf) != 0);
-    if (P->qp_far) { gs = 64; P->staged = 0; P->smem_qp = 0; }
-    P->gs_qp = gs;
+    const int qp_far = (P->staged ? with_state : without) > budget || (qpf && atoi(qpf) != 0);
+    if (qp_far) { gs = 64; P->staged = 0; }
+    P->qp = {gs, qp_far, qp_far ? 0 : P->staged ? with_state : without};
     // (a state of tens of MB per problem -- 3-D, N = 512 -- makes chunks of fewer than 1024 problems: the cap holds)
     size_t chunk = TG_PHASED_CHUNK_BYTES / (P->np * sizeof(double));
     if (chunk < 1) chunk = 1;
@@ -256,27 +248,45 @@ static int tg_plan_solve(const TgShape &S, int B, TgSolvePlan *P)
     P->chunk = (int)chunk;
     P->phased_bytes = chunk * P->np * sizeof(double);
     // workspace slots: one per lane group of a grid capped at TG_FAR_CTAS_PER_SM CTAs per SM and at the chunk's work
-    // (far-placed shapes run as one slice: tg_solve_phased)
     auto slots_of = [&](int groups) {
         const size_t need = (chunk + groups - 1) / groups, cap = (size_t)g_sm_count * TG_FAR_CTAS_PER_SM;
         return (need < cap ? need : cap) * groups;
     };
-    const size_t qp_slots = P->qp_far ? slots_of(128 / 64) : 0, ls_slots = P->ls_far ? slots_of(128 / 32) : 0;
-    const size_t qp_bytes = qp_slots * tg_sqp_qp_scratch_doubles(S.L) * sizeof(double);
-    const size_t ls_bytes = ls_slots * tg_sqp_ls_slot_doubles(S.L) * sizeof(double);
+    const size_t qp_slots = qp_far ? slots_of(TG_CTA_THREADS / 64) : 0, ls_slots = ls_far ? slots_of(TG_CTA_THREADS / 32) : 0;
+    const size_t qp_bytes = qp_slots * tg_sqp_qp_scratch_doubles(L) * sizeof(double);
+    const size_t ls_bytes = ls_slots * tg_sqp_ls_slot_doubles(L) * sizeof(double);
     P->slots = (int)(qp_slots > ls_slots ? qp_slots : ls_slots);
     P->slot_bytes = ((qp_bytes > ls_bytes ? qp_bytes : ls_bytes) + 255) & ~(size_t)255;
+    // slices: measured on B200 (65,536 problems): two slices -9.5 % on C2 (short stage kernels, a long tail of rounds
+    // with few problems), -2 % on C3, +3 % on C5a, +8 % on C4 (state in L2 / HBM): two when the state is staged in shared
+    // memory.  Far-placed shapes run as one slice: the workspace slots serve one grid at a time.
+    P->slices = P->staged ? 2 : 1;
+    if (const char *v = getenv("TG_SLICES")) P->slices = atoi(v);
+    if (P->slot_bytes) P->slices = 1;
+    if (P->slices < 1) P->slices = 1;
+    if (P->slices > TG_MAX_SLICES) P->slices = TG_MAX_SLICES;
     return 0;
 }
 
-static size_t tg_lists_bytes(int chunk);
+// device bookkeeping in front of the per-problem state: [TgRoundCtl x TG_MAX_SLICES | list0[chunk] | list1[chunk] |
+// workspace slots (far-placed stages only)]
+#define TG_HEADER_BYTES (TG_MAX_SLICES * TG_ROUNDCTL_BYTES)
+static size_t tg_lists_bytes(int chunk) { return (((size_t)2 * chunk * sizeof(int)) + 255) & ~(size_t)255; }
+
+// bytes of the solve workspace: the lock-step solve's, or the fused kernel's global workspace where that is larger
+static size_t tg_workspace_bytes(const TgShape &S, int B, const TgSolvePlan &P)
+{
+    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk) + P.slot_bytes;
+    const size_t fused = tg_fused_workspace_bytes(S, B, g_sm_count, g_smem_optin);
+    return (fused > phased ? fused : phased) + TG_HEADER_BYTES;
+}
+
 extern "C" size_t tg_solve_workspace_bytes(const int *spec, int B)
 {
     TgShape S;
     TgSolvePlan P;
     if (tg_make_shape(spec, &S) || tg_plan_solve(S, B, &P)) return 0;
-    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk) + P.slot_bytes;
-    return (P.global_bytes > phased ? P.global_bytes : phased) + 4 * TG_ROUNDCTL_BYTES;
+    return tg_workspace_bytes(S, B, P);
 }
 
 extern "C" int tg_solve_plan_info(const int *spec, int B, int *out, int cap)
@@ -286,7 +296,7 @@ extern "C" int tg_solve_plan_info(const int *spec, int B, int *out, int cap)
     int rc = tg_make_shape(spec, &S);
     if (!rc) rc = tg_plan_solve(S, B > 0 ? B : 1, &P);
     if (rc) return -rc;
-    const int v[7] = {P.gs_ls, P.gs_qp, P.staged, P.qp_far, P.ls_far, P.slots, (int)(P.slot_bytes >> 10)};
+    const int v[7] = {P.ls.lanes, P.qp.lanes, P.staged, P.qp.far, P.ls.far, P.slots, (int)(P.slot_bytes >> 10)};
     for (int i = 0; i < 7 && out && i < cap; i++) out[i] = v[i];
     return 7;
 }
@@ -320,15 +330,9 @@ extern "C" int tg_last_solve_stats(double *out, int cap)
     return 6;
 }
 
-// device bookkeeping in front of the per-problem state: [TgRoundCtl x TG_MAX_SLICES | list0[chunk] | list1[chunk] |
-// workspace slots (far-placed stages only)]
-#define TG_MAX_SLICES 4
-#define TG_HEADER_BYTES (TG_MAX_SLICES * TG_ROUNDCTL_BYTES)
-static size_t tg_lists_bytes(int chunk) { return (((size_t)2 * chunk * sizeof(int)) + 255) & ~(size_t)255; }
-
-// A chunk is solved as up to TG_MAX_SLICES independent slices, each with its own round bookkeeping and its own
-// stream: while one slice's stage kernel drains (a round lasts as long as its slowest problem), the other slices'
-// kernels fill the machine.  TG_SLICES overrides the count; stage timing runs one slice (unoverlapped kernels).
+// A chunk is solved as up to TG_MAX_SLICES independent slices (the plan's count), each with its own round bookkeeping
+// and its own stream: while one slice's stage kernel drains (a round lasts as long as its slowest problem), the other
+// slices' kernels fill the machine.  Stage timing runs one slice (unoverlapped kernels).
 struct TgSliceStreams {
     cudaStream_t st[TG_MAX_SLICES] = {nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t fork = nullptr, join[TG_MAX_SLICES] = {nullptr, nullptr, nullptr, nullptr};
@@ -373,6 +377,16 @@ struct TgSliceLease {
     }
 };
 
+// the plan's stage: its launcher for its lanes, its shared memory and slots
+static cudaError_t tg_launch_stage(const TgStageLauncher launchers[4], const TgStagePlan &s, TgStageLaunch &a, double *slots)
+{
+    a.smem = s.smem;
+    a.far = s.far ? slots : nullptr;
+    const TgStageLauncher launch = launchers[tg_lanes_index(s.lanes)];
+    assert(launch);
+    return launch(a);
+}
+
 static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const double *par, double *x, double *f,
                            int *status, int *nit, int *violation, int maxiter, double ftol, int flags, void *workspace,
                            cudaStream_t st)
@@ -380,9 +394,8 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
     const TgLayout &L = S.L;
     char *wsb = (char *)workspace;
     int *list_base = (int *)(wsb + TG_HEADER_BYTES);
-    double *far = (double *)(wsb + TG_HEADER_BYTES + tg_lists_bytes(P.chunk));
-    double *pws_base = (double *)((char *)far + P.slot_bytes);
-    double *far_qp = P.qp_far ? far : nullptr, *far_ls = P.ls_far ? far : nullptr;
+    double *slots = (double *)(wsb + TG_HEADER_BYTES + tg_lists_bytes(P.chunk));
+    double *pws_base = (double *)((char *)slots + P.slot_bytes);
     const bool timing = g_stage_timing.load() != 0;
     std::vector<cudaEvent_t> ev;
     if (timing) g_stats = TgSolveStats{0, 0, 0, 0, 0, 0};
@@ -394,17 +407,10 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
         ev.push_back(e);
         return cudaEventRecord(e, st);
     };
-    // measured on B200 (65,536 problems): two slices -9.5 % on C2 (short stage kernels, a long tail of rounds with few
-    // problems), -2 % on C3, +3 % on C5a, +8 % on C4 (state in L2 / HBM): two when the state is staged in shared memory
-    int want = P.staged ? 2 : 1;
-    if (const char *v = getenv("TG_SLICES")) want = atoi(v);
-    if (P.slot_bytes) want = 1;          // the workspace slots serve one grid at a time
-    if (want < 1) want = 1;
-    if (want > TG_MAX_SLICES) want = TG_MAX_SLICES;
     TgSliceLease lease;
     for (int lo = 0; lo < B; lo += P.chunk) {
         const int nbc = B - lo < P.chunk ? B - lo : P.chunk;
-        const int ns = (timing || nbc < 8192) ? 1 : want;
+        const int ns = (timing || nbc < 8192) ? 1 : P.slices;
         if (ns > 1) {
             TG_CUDA(lease.acquire());
             TG_CUDA(cudaEventRecord(lease.s->fork, st));
@@ -435,22 +441,13 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
                 Slice &q = sl[k];
                 if (q.done >= q.nb) continue;
                 any = true;
-                const double *cpar = par + (size_t)(lo + q.lo) * L.P;
+                TgStageLaunch a = {S, q.nb, par + (size_t)(lo + q.lo) * L.P, q.pws, P.np, 0, nullptr, P.staged, q.rc,
+                                   q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, P.fix, q.st};
                 TG_CUDA(mark());
-                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_ls_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                      tg_launch_ls_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                      tg_launch_ls_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
-                          "tg_sqp_ls_kernel");
-                TG_LAUNCH(TG_DISPATCH(P.gs_ls, tg_launch_fd_g8(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                          tg_launch_fd_g16(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st),
-                                          tg_launch_fd_g32(S, q.nb, cpar, q.pws, P.np, P.smem_ls, far_ls, q.rc, q.lists[par_], par_, g_sm_count, q.st)),
-                          "tg_sqp_der_kernel");
+                TG_LAUNCH(tg_launch_stage(tg_ls_launchers, P.ls, a, slots), "tg_sqp_ls_kernel");
+                TG_LAUNCH(tg_launch_stage(tg_fd_launchers, P.der, a, slots), "tg_sqp_der_kernel");
                 TG_CUDA(mark());
-                TG_LAUNCH(P.gs_qp == 64 ? tg_launch_qp_g64(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st) :
-                          TG_DISPATCH(P.gs_qp, tg_launch_qp_g8(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
-                                      tg_launch_qp_g16(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st),
-                                      tg_launch_qp_g32(S, q.nb, q.pws, P.np, P.staged, P.smem_qp, far_qp, q.rc, q.lists[par_], q.lists[par_ ^ 1], par_, g_sm_count, q.st)),
-                          "tg_sqp_qp_kernel");
+                TG_LAUNCH(tg_launch_stage(tg_qp_launchers, P.qp, a, slots), "tg_sqp_qp_kernel");
                 TG_CUDA(mark());
             }
             if (!any) break;
@@ -504,17 +501,13 @@ extern "C" int tg_solve_batch(const int *spec, int B, const double *par, double 
     if (rc) return rc;
     if (B <= 0) return 0;
     if ((rc = tg_plan_solve(S, B, &P))) return rc;
-    const size_t phased = P.phased_bytes + tg_lists_bytes(P.chunk) + P.slot_bytes;
-    const size_t need = (P.global_bytes > phased ? P.global_bytes : phased) + TG_HEADER_BYTES;
-    if (!workspace || workspace_bytes < need) return tg_fail(4, "workspace too small (see tg_solve_workspace_bytes)");
-    int *counters = (int *)workspace;
-    double *gws = (double *)((char *)workspace + 256);
+    if (!workspace || workspace_bytes < tg_workspace_bytes(S, B, P)) return tg_fail(4, "workspace too small (see tg_solve_workspace_bytes)");
     cudaStream_t st = (cudaStream_t)stream;
     if (flags & TG_SOLVE_FUSED) {
+        int *counters = (int *)workspace;
         TG_CUDA(cudaMemsetAsync(counters, 0, 256, st));
-        TG_LAUNCH(tg_launch_fused_g32(S, B, par, x, f, status, nit, violation, maxiter, ftol, flags,
-                                      P.use_global ? gws : nullptr, P.ws_doubles, P.warps_per_cta, P.ctas, P.smem_bytes,
-                                      counters, st), "tg_solve_kernel");
+        TG_LAUNCH(tg_launch_fused_g32(S, B, par, x, f, status, nit, violation, maxiter, ftol, flags, (char *)workspace + 256,
+                                      counters, g_sm_count, g_smem_optin, st), "tg_solve_kernel");
         return 0;
     }
     return tg_solve_phased(S, P, B, par, x, f, status, nit, violation, maxiter, ftol, flags, workspace, st);

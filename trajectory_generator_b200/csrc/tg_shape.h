@@ -1,4 +1,5 @@
-// Shared between the host API (tg_api.cu) and the per-group-size kernel translation units.
+// Shared between the host API (tg_api.cu) and the per-group-size kernel translation units: the shape a kernel is
+// launched for, the fixed shapes with instantiations of their own, and the launchers with their arguments.
 #ifndef TG_SHAPE_H
 #define TG_SHAPE_H
 #include <cuda_runtime.h>
@@ -108,46 +109,56 @@ static inline cudaError_t tg_allow_shared_memory(K kernel)
     return cudaSuccess;
 }
 
-#define TG_DECLARE_VARIANT(SFX)                                                                                           \
-    cudaError_t tg_launch_eval##SFX(const TgShape &S, int B, const double *par, const double *x, double *f, double *g,    \
-                                    double *c, double *jnl, int sm_count, int smem_optin, cudaStream_t st);               \
-    cudaError_t tg_launch_linear##SFX(const TgShape &S, int B, const double *par, double *alin, int sm_count,             \
-                                      cudaStream_t st);                                                                   \
-    size_t tg_eval_smem##SFX(const TgShape &S, bool sink_c, int smem_optin);                                              \
-    cudaError_t tg_launch_begin##SFX(const TgShape &S, int B, const double *x, double *pws, size_t np, int maxiter,       \
-                                     double ftol, int flags, TgRoundCtl *rc, int *list0, cudaStream_t st);                \
-    cudaError_t tg_launch_ls##SFX(const TgShape &S, int B, const double *par, double *pws, size_t np, size_t smem,        \
-                                  double *far, TgRoundCtl *rc, const int *list, int parity, int sm_count,                 \
-                                  cudaStream_t st);                                                                       \
-    cudaError_t tg_launch_qp##SFX(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem, double *far,  \
-                                  TgRoundCtl *rc, const int *list, int *next, int parity, int sm_count, cudaStream_t st); \
-    size_t tg_ls_smem##SFX(const TgShape &S);                                                                             \
-    size_t tg_qp_smem##SFX(const TgShape &S, int staged);                                                                 \
-    cudaError_t tg_launch_finish##SFX(const TgShape &S, int B, const double *pws, size_t np, double *x, double *f,        \
-                                      int *status, int *nit, int *violation, TgRoundCtl *rc, cudaStream_t st);
+// Launchers of the device code (per lanes per problem: the tg_*_g<lanes>.cu translation units).  The host plan
+// (tg_api.cu: tg_plan_solve, tg_eval_batch) decides every launch parameter; a launcher picks the instantiation for the
+// fixed-shape index, the dimension and the placement it is handed and launches it.
+//
+// Lock-step stage kernels (tg_kernels_solve.inc).  tg_solve_phased fills one TgStageLaunch per slice and round and sets
+// the stage's shared memory and workspace slots (far != nullptr: scratch in global memory) before each launch.
+struct TgStageLaunch {
+    TgShape S;
+    int B;                  // problems of the slice (the grids are capped at the work)
+    const double *par;      // parameter rows of the slice
+    double *pws;            // persistent state of the slice's problems, np doubles each
+    size_t np;
+    size_t smem;            // dynamic shared memory of the stage's CTAs
+    double *far;            // workspace slots of the stage, or nullptr
+    int staged;             // QP stage: the persistent state is staged through shared memory
+    TgRoundCtl *rc;
+    const int *list;        // this round's list of unfinished problems
+    int *next;              // QP stage: the next round's list
+    int parity;             // round & 1
+    int sm_count, fix;      // fix: tg_fixed_index of the shape, 0 = generic instantiations
+    cudaStream_t st;
+};
+cudaError_t tg_launch_ls_g8(const TgStageLaunch &a), tg_launch_ls_g16(const TgStageLaunch &a), tg_launch_ls_g32(const TgStageLaunch &a);
+cudaError_t tg_launch_fd_g8(const TgStageLaunch &a), tg_launch_fd_g16(const TgStageLaunch &a), tg_launch_fd_g32(const TgStageLaunch &a);
+cudaError_t tg_launch_qp_g16(const TgStageLaunch &a), tg_launch_qp_g32(const TgStageLaunch &a), tg_launch_qp_g64(const TgStageLaunch &a);
+// once per solve (32 lanes)
+cudaError_t tg_launch_begin_g32(const TgShape &S, int B, const double *x, double *pws, size_t np, int maxiter, double ftol,
+                                int flags, TgRoundCtl *rc, int *list0, cudaStream_t st);
+cudaError_t tg_launch_finish_g32(const TgShape &S, int B, const double *pws, size_t np, double *x, double *f, int *status,
+                                 int *nit, int *violation, TgRoundCtl *rc, cudaStream_t st);
 
-TG_DECLARE_VARIANT(_g8)
-TG_DECLARE_VARIANT(_g16)
-TG_DECLARE_VARIANT(_g32)
-
-// finite-difference stage (tg_solve_fd_g*.cu): value-only evaluators inlined, one kernel of its own
-#define TG_DECLARE_FD(SFX)                                                                                              \
-    cudaError_t tg_launch_fd##SFX(const TgShape &S, int B, const double *par, double *pws, size_t np, size_t smem,      \
-                                  double *far, TgRoundCtl *rc, const int *list, int parity, int sm_count, cudaStream_t st);
-TG_DECLARE_FD(_g8)
-TG_DECLARE_FD(_g16)
-TG_DECLARE_FD(_g32)
-
-// QP stage with 64 lanes per problem (tg_solve_g64.cu)
-cudaError_t tg_launch_qp_g64(const TgShape &S, int B, double *pws, size_t np, int staged, size_t smem, double *far,
-                             TgRoundCtl *rc, const int *list, int *next, int parity, int sm_count, cudaStream_t st);
-size_t tg_qp_smem_g64(const TgShape &S, int staged);
+// Evaluation kernel (tg_kernels_eval.inc): `groups` lane groups per CTA with `smem` bytes of shared memory
+struct TgEvalLaunch {
+    TgShape S;
+    int B;
+    const double *par, *x;
+    double *f, *g, *c, *jnl;
+    int fix, grid, groups;
+    size_t smem;
+    cudaStream_t st;
+};
+cudaError_t tg_launch_eval_g8(const TgEvalLaunch &a), tg_launch_eval_g16(const TgEvalLaunch &a), tg_launch_eval_g32(const TgEvalLaunch &a);
+cudaError_t tg_launch_linear_g32(const TgShape &S, int B, const double *par, double *alin, int sm_count, cudaStream_t st);
 
 // launch counter of the library (tg_launch_count), for kernels launched outside tg_api.cu
 void tg_note_launch(int count);
 
-// fused kernel (group size 32 only)
+// fused kernel (tg_solve_fused.cu, 32 lanes): it sizes its grid and its global workspace itself (the same numbers for both)
+size_t tg_fused_workspace_bytes(const TgShape &S, int B, int sm_count, int smem_optin);
 cudaError_t tg_launch_fused_g32(const TgShape &S, int B, const double *par, double *x, double *f, int *status, int *nit,
-                                int *violation, int maxiter, double ftol, int flags, double *gws, size_t ws_doubles,
-                                int warps_per_cta, int ctas, size_t smem, int *queue, cudaStream_t st);
+                                int *violation, int maxiter, double ftol, int flags, void *gws, int *queue, int sm_count,
+                                int smem_optin, cudaStream_t st);
 #endif

@@ -2,6 +2,6 @@
 // with the evaluators inlined value-only (see tg_kernels_solve.inc)
 #define TG_GS 32
 #define TG_INLINE_ALL
-#define TG_FD_ONLY
+#define TG_DER_STAGE
 #define TG_SFX _g32
 #include "tg_kernels_solve.inc"

@@ -48,19 +48,61 @@ tg_solve_kernel(const TgShape S, int B, const double *__restrict__ par, double *
     }
 }
 
-cudaError_t tg_launch_fused_g32(const TgShape &S, int B, const double *par, double *x, double *f, int *status, int *nit,
-                                int *violation, int maxiter, double ftol, int flags, double *gws, size_t ws_doubles,
-                                int warps_per_cta, int ctas, size_t smem, int *queue, cudaStream_t st)
+// grid and workspace of the fused kernel: a shared-memory workspace per warp when at least 8 warps fit on an SM, else
+// a global one (per resident warp) in the solve workspace
+struct TgFusedPlan {
+    int warps_per_cta, ctas, use_global;
+    size_t ws_doubles, smem_bytes, global_bytes;
+};
+
+static TgFusedPlan tg_fused_plan(const TgShape &S, int B, int sm_count, int smem_optin)
 {
+    TgFusedPlan P;
+    const size_t budget = (size_t)smem_optin - 1024;
+    const size_t sm_total = 227 * 1024;
+    P.ws_doubles = tg_sqp_workspace_doubles(S.L);
+    const size_t per_warp_shared = (S.L.P + P.ws_doubles + 2) * sizeof(double);
+    if (per_warp_shared * 8 <= sm_total) {
+        P.use_global = 0;
+        P.warps_per_cta = 4;
+        while (per_warp_shared * P.warps_per_cta > budget) P.warps_per_cta >>= 1;
+        P.smem_bytes = per_warp_shared * P.warps_per_cta;
+        int per_sm = (int)(sm_total / (P.smem_bytes + 1024));
+        if (per_sm < 1) per_sm = 1;
+        if (per_sm * P.warps_per_cta > 32) per_sm = 32 / P.warps_per_cta;
+        P.ctas = sm_count * per_sm;
+    } else {
+        P.use_global = 1;
+        P.warps_per_cta = 4;
+        P.smem_bytes = (size_t)P.warps_per_cta * (S.L.P + 2) * sizeof(double);
+        P.ctas = sm_count * 4;
+    }
+    const int need = (B + P.warps_per_cta - 1) / P.warps_per_cta;
+    if (P.ctas > need) P.ctas = need > 0 ? need : 1;
+    P.global_bytes = P.use_global ? (size_t)P.ctas * P.warps_per_cta * P.ws_doubles * sizeof(double) : 0;
+    return P;
+}
+
+size_t tg_fused_workspace_bytes(const TgShape &S, int B, int sm_count, int smem_optin)
+{
+    return tg_fused_plan(S, B, sm_count, smem_optin).global_bytes;
+}
+
+cudaError_t tg_launch_fused_g32(const TgShape &S, int B, const double *par, double *x, double *f, int *status, int *nit,
+                                int *violation, int maxiter, double ftol, int flags, void *gws, int *queue, int sm_count,
+                                int smem_optin, cudaStream_t st)
+{
+    const TgFusedPlan P = tg_fused_plan(S, B, sm_count, smem_optin);
+    double *ws = P.use_global ? (double *)gws : nullptr;
     cudaError_t e;
     if (S.L.d == 2) {
         if ((e = tg_allow_shared_memory(tg_solve_kernel<2>))) return e;
-        tg_solve_kernel<2><<<ctas, warps_per_cta * 32, smem, st>>>(S, B, par, x, f, status, nit, violation, maxiter, ftol,
-                                                                    flags, gws, ws_doubles, warps_per_cta, queue);
+        tg_solve_kernel<2><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, maxiter,
+                                                                                ftol, flags, ws, P.ws_doubles, P.warps_per_cta, queue);
     } else {
         if ((e = tg_allow_shared_memory(tg_solve_kernel<3>))) return e;
-        tg_solve_kernel<3><<<ctas, warps_per_cta * 32, smem, st>>>(S, B, par, x, f, status, nit, violation, maxiter, ftol,
-                                                                    flags, gws, ws_doubles, warps_per_cta, queue);
+        tg_solve_kernel<3><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, maxiter,
+                                                                                ftol, flags, ws, P.ws_doubles, P.warps_per_cta, queue);
     }
     return cudaGetLastError();
 }

@@ -258,6 +258,39 @@ TG_HD size_t tg_sqp_persistent_doubles(const TgLayout &L) { size_t a, b; tg_sqp_
 TG_HD size_t tg_sqp_scratch_doubles(const TgLayout &L) { size_t a, b; tg_sqp_carve2(L, 0, 0, 0, &a, &b); return b; }
 TG_HD size_t tg_sqp_workspace_doubles(const TgLayout &L) { return tg_sqp_persistent_doubles(L) + tg_sqp_scratch_doubles(L); }
 
+// Shared memory of the lock-step stage kernels and the evaluation kernel (tg_kernels_solve.inc, tg_kernels_eval.inc):
+// a CTA of TG_CTA_THREADS threads holds TG_CTA_THREADS / lanes lane groups.
+#define TG_CTA_THREADS 128
+// line-search / derivative stage, per lane group: [parameters | state prefix | evaluation scratch], every piece starting
+// on a 16-byte boundary (the derivative stage stages the shorter prefix, tg_sqp_prefix_fd_doubles)
+TG_HD size_t tg_ls_par_doubles(const TgLayout &L) { return ((size_t)L.P + 2) & ~(size_t)1; }
+TG_HD size_t tg_ls_group_doubles(const TgLayout &L)
+{
+    const size_t n = tg_ls_par_doubles(L) + tg_sqp_prefix_doubles(L) + tg_sqp_ls_scratch_doubles(L);
+    return n + (n & 1);
+}
+TG_HD size_t tg_fd_group_doubles(const TgLayout &L)
+{
+    const size_t n = tg_ls_par_doubles(L) + tg_sqp_prefix_fd_doubles(L) + tg_sqp_ls_scratch_doubles(L);
+    return n + (n & 1);
+}
+TG_HD size_t tg_ls_smem_bytes(const TgLayout &L, int lanes) { return (size_t)(TG_CTA_THREADS / lanes) * tg_ls_group_doubles(L) * sizeof(double); }
+TG_HD size_t tg_fd_smem_bytes(const TgLayout &L, int lanes) { return (size_t)(TG_CTA_THREADS / lanes) * tg_fd_group_doubles(L) * sizeof(double); }
+// QP stage: the scratch, and with `staged` the persistent state except the factor L (which stays in global memory)
+TG_HD size_t tg_qp_smem_bytes(const TgLayout &L, int lanes, int staged)
+{
+    const size_t state = staged ? tg_sqp_persistent_doubles(L) - tg_sqp_factor_doubles(L) : 0;
+    return (size_t)(TG_CTA_THREADS / lanes) * (tg_sqp_qp_scratch_doubles(L) + state) * sizeof(double);
+}
+// evaluation kernel: lane groups of one CTA -- TG_CTA_THREADS / lanes, fewer where their shared memory exceeds the
+// opt-in limit (long trajectories: 3-D with 8 x 63 corridor intervals needs 163 KB a group without `c`), 0 where not
+// even one group fits
+TG_HD int tg_eval_groups(const TgLayout &L, int lanes, bool sink_c, int smem_optin)
+{
+    const size_t fit = (size_t)smem_optin / (tg_eval_group_doubles(L, sink_c) * sizeof(double));
+    return fit < (size_t)(TG_CTA_THREADS / lanes) ? (int)fit : TG_CTA_THREADS / lanes;
+}
+
 // one contiguous buffer: persistent part first, scratch behind it
 TG_HD size_t tg_sqp_carve(const TgLayout &L, double *base, TgSqpWs *W)
 {
