@@ -110,6 +110,33 @@ int tg_solve_mixed_batch(int nbuckets, const int *specs, const int *counts, cons
                          double ftol, int flags, void *stream);
 
 /*
+ * Multi-start solves: K seeded starts per problem, solved as ordinary problems, the best one kept.  The problems are
+ * non-convex and SLSQP converges to the basin its start lies in; several starts find better basins.  A multi-start
+ * solve of B problems is three calls on one stream:
+ *   tg_multistart_expand  par[B*P], x0[B*n] -> par_out[B*K*P], x_out[B*K*n]: row b*K + k is start k of problem b.
+ *       par_out rows are copies of par[b].  Start 0 is x0[b] bit for bit (K = 1 is an ordinary solve).  Start k > 0
+ *       offsets the interior control points (3 .. N-4 of each coordinate) by spread * |P_{N-1} - P_0| times a smooth
+ *       profile drawn from a splitmix64 hash of (seed, k, coordinate, knot), and multiplies the scale factor by
+ *       1, 1/2, 2, 3/4, 3/2, 5/8, 5/4, 3 (k mod 8); waypoint scalars and intermediate times are copied
+ *       (csrc/tg_multistart.cu).  The starts depend on (seed, k) and on the problem itself, never on b.
+ *   tg_solve_batch / tg_solve_mixed_batch on the B*K rows, unchanged.
+ *   tg_multistart_select  per problem, the constraint rows at each start's final point xs[B*K*n] are folded into the
+ *       true maximum violation (max |c| over the equality rows, max(0, -c) over the inequality rows, NaN = +inf;
+ *       written to max_violation[B*K] unless it is NULL).  The winner: a start with status 0 and maximum violation
+ *       <= tol beats every other start, the lowest f among them (NaN = +inf); with no such start, the lowest maximum
+ *       violation, then the lowest f; remaining ties go to the lowest k.  Its x / f / status / nit / violation are
+ *       gathered into x_best[B*n], f_best[B], status_best[B], nit_best[B], violation_best[B] (violation stays the
+ *       reference's is_violation flag) and best_start[b] = k.  par[B*P] are the B problems' rows.
+ * Device pointers; K >= 1.  Returns 0, or an error code with tg_last_error() (K < 1, NULL required pointer, no device).
+ */
+int tg_multistart_expand(const int *spec, int B, int K, const double *par, const double *x0, unsigned long long seed,
+                         double spread, double *par_out, double *x_out, void *stream);
+int tg_multistart_select(const int *spec, int B, int K, const double *par, const double *xs, const double *f,
+                         const int *status, const int *nit, const int *violation, double tol, double *x_best,
+                         double *f_best, int *status_best, int *nit_best, int *violation_best, int *best_start,
+                         double *max_violation, void *stream);
+
+/*
  * Output sampling of a batch of cubic trajectories (SURVEY.md 8(f) f1), device pointers:
  *   mode 0: matrix_bspline_evaluation_for_dataset / matrix_bspline_derivative_evaluation_for_dataset
  *           (TG/matrix_evaluation.py:5-33, 104-135): num_points samples over the N-3 intervals of every trajectory;

@@ -26,7 +26,7 @@ LAYOUT_FIELDS = ("d N nint n ia is0 is1 it0 nws niw meq mineq m r_start n_start 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 # translation units: the host API (+ legacy single-problem kernels) and one unit per (kernel family, lanes per problem)
-UNITS = ["tg_api.cu", "tg_sample.cu", "tg_build.cu", "tg_smooth.cu", "tg_solve_fused.cu", "tg_solve_g64.cu"] + ["tg_%s_g%d.cu" % (fam, gs) for fam in ("eval", "solve", "solve_fd") for gs in (8, 16, 32)]
+UNITS = ["tg_api.cu", "tg_sample.cu", "tg_build.cu", "tg_smooth.cu", "tg_multistart.cu", "tg_solve_fused.cu", "tg_solve_g64.cu"] + ["tg_%s_g%d.cu" % (fam, gs) for fam in ("eval", "solve", "solve_fd") for gs in (8, 16, 32)]
 HEADERS = ["tg_sqp.h", "tg_eval.h", "tg_spec.h", "tg_shape.h", "tg_smooth.h", "tg_kernels_eval.inc", "tg_kernels_solve.inc"]
 
 
@@ -128,6 +128,10 @@ def lib():
         L.tg_initial_guess_batch.restype = ctypes.c_int
         L.tg_sfc_boxes_batch.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp]
         L.tg_sfc_boxes_batch.restype = ctypes.c_int
+        L.tg_multistart_expand.argtypes = [_I32, ctypes.c_int, ctypes.c_int, vp, vp, ctypes.c_uint64, ctypes.c_double, vp, vp, vp]
+        L.tg_multistart_expand.restype = ctypes.c_int
+        L.tg_multistart_select.argtypes = [_I32, ctypes.c_int, ctypes.c_int] + [vp] * 6 + [ctypes.c_double] + [vp] * 8
+        L.tg_multistart_select.restype = ctypes.c_int
         for name in ("tg_eval_batch", "tg_linear_rows_batch", "tg_solve_batch", "tg_eval_host", "tg_solve_host"):
             getattr(L, name).restype = ctypes.c_int
         _LIB = L

@@ -5,7 +5,8 @@ host-buffer (numpy, copies inside the C call) variants of
     rows of the nonlinear constraints, for B problems of one shape; what the reference computes with
     1 + (n+1) Python calls of every closure per SLSQP iteration (TG/trajectory_generator.py:171-250
     under scipy's finite differences);
-  * ``solve``     -- M2: the scipy SLSQP call of TG/trajectory_generator.py:87-94 for B problems.
+  * ``solve``     -- M2: the scipy SLSQP call of TG/trajectory_generator.py:87-94 for B problems;
+  * ``solve_multistart`` -- M2 from K seeded starts per problem, the best converged feasible result kept (opt-in).
 
 PyTorch is used only to own device memory and streams.
 """
@@ -268,3 +269,144 @@ def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
                                     _stream(torch, dev))
     _native.check(rc, "tg_solve_mixed_batch")
     return outs
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Multi-start solves (include/trajectory_generator_b200.h, DESIGN.md §4 *Multi-start*): K seeded starts per problem are
+# solved as ordinary problems and the best converged feasible one is kept.
+# ---------------------------------------------------------------------------------------------------------------------
+MULTISTART_SPREAD = 0.25    # offset scale of the interior control points, relative to |P_{N-1} - P_0| (DESIGN.md §4)
+MULTISTART_TOL = 1e-5       # feasibility tolerance of the selection: the reference's is_violation tolerance (10e-6)
+MULTISTART_ROWS = 1 << 20   # cap of the B * K rows expanded at a time (par is replicated: B * K * P doubles)
+
+
+def _check_device_rows(what, spec, par, x, starts=1):
+    """(layout, B) of par [B, P] and x [B * starts, n]: contiguous float64 CUDA tensors on one device"""
+    torch = _torch()
+    lay = Layout(spec)
+    if not (par.is_cuda and x.is_cuda):
+        raise RuntimeError("%s needs CUDA tensors (there is no CPU path)" % what)
+    if par.dtype != torch.float64 or x.dtype != torch.float64:
+        raise ValueError("%s needs float64 tensors, got %s / %s" % (what, par.dtype, x.dtype))
+    if par.device != x.device:
+        raise ValueError("par and x live on different devices")
+    B = par.shape[0]
+    if not (par.is_contiguous() and x.is_contiguous()) or par.shape != (B, lay.P) or x.shape != (B * starts, lay.n):
+        raise ValueError("par [B, %d] and x [B * %d, %d] must be contiguous tensors of the descriptor's shape"
+                         % (lay.P, starts, lay.n))
+    return lay, B
+
+
+def multistart_expand(spec, par, x0, starts, seed=0, spread=MULTISTART_SPREAD):
+    """Starts of B problems (tg_multistart_expand): par [B, P], x0 [B, n] float64 CUDA tensors ->
+    (par_out [B*K, P], x_out [B*K, n]); row b*K + k is start k of problem b, start 0 is x0[b] bit for bit."""
+    torch = _torch()
+    lay, B = _check_device_rows("multistart_expand()", spec, par, x0)
+    K = int(starts)
+    if K < 1:
+        raise ValueError("starts must be at least 1")
+    dev = x0.device
+    par_out = torch.empty((B * K, lay.P), dtype=torch.float64, device=dev)
+    x_out = torch.empty((B * K, lay.n), dtype=torch.float64, device=dev)
+    spec, sp = _native.spec_ptr(spec)
+    with torch.cuda.device(dev):
+        rc = _native.lib().tg_multistart_expand(sp, B, K, _ptr(par), _ptr(x0), int(seed) & (2 ** 64 - 1), float(spread),
+                                                _ptr(par_out), _ptr(x_out), _stream(torch, dev))
+    _native.check(rc, "tg_multistart_expand")
+    return par_out, x_out
+
+
+def multistart_select(spec, par, sol, starts, tol=MULTISTART_TOL, out=None):
+    """Best start per problem (tg_multistart_select).  par [B, P]: the problems' rows; sol: the dict a solve of the
+    B*K expanded rows returned.  Returns dict(x, f, status, nit, violation, best_start, max_violation) with B rows and
+    `start_max_violation` [B, K] (the true maximum violation of every start); `out` may hold any of these to write into."""
+    torch = _torch()
+    K = int(starts)
+    if K < 1:
+        raise ValueError("starts must be at least 1")
+    lay, B = _check_device_rows("multistart_select()", spec, par, sol["x"], K)
+    dev = par.device
+    res = {} if out is None else out
+    shapes = dict(x=((B, lay.n), torch.float64), f=((B,), torch.float64), status=((B,), torch.int32),
+                  nit=((B,), torch.int32), violation=((B,), torch.int32), best_start=((B,), torch.int32),
+                  start_max_violation=((B, K), torch.float64))
+    for k, (shape, dtype) in shapes.items():
+        if k not in res:
+            res[k] = torch.empty(shape, dtype=dtype, device=dev)
+    spec, sp = _native.spec_ptr(spec)
+    with torch.cuda.device(dev):
+        rc = _native.lib().tg_multistart_select(
+            sp, B, K, _ptr(par), _ptr(sol["x"]), _ptr(sol["f"]), _ptr(sol["status"]), _ptr(sol["nit"]),
+            _ptr(sol["violation"]), float(tol), _ptr(res["x"]), _ptr(res["f"]), _ptr(res["status"]), _ptr(res["nit"]),
+            _ptr(res["violation"]), _ptr(res["best_start"]), _ptr(res["start_max_violation"]), _stream(torch, dev))
+    _native.check(rc, "tg_multistart_select")
+    res["max_violation"] = res["start_max_violation"].gather(1, res["best_start"].long()[:, None])[:, 0]
+    return res
+
+
+def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100,
+                           ftol=1e-6, jacobian="analytic", return_all=False):
+    """Multi-start solve of problems of one or several shapes: buckets = list of (spec, par [Bk, P], x0 [Bk, n]) CUDA
+    tensors (x0 is not modified).  Per bucket: expand -> solve -> select on the current stream, in pieces of at most
+    MULTISTART_ROWS expanded rows; the pieces of several shapes go through one ``solve_mixed`` call.  Returns one dict
+    per bucket: the B-row dict of ``solve`` plus best_start and max_violation (the winner's true maximum violation);
+    with return_all, also "all": the K per-start results, dict(x [B, K, n], f, status, nit, violation,
+    max_violation [B, K])."""
+    torch = _torch()
+    K = int(starts)
+    if K < 1:
+        raise ValueError("starts must be at least 1")
+    outs, pieces = [], []
+    for j, (spec, par, x0) in enumerate(buckets):
+        lay, B = _check_device_rows("solve_multistart()", spec, par, x0)
+        dev = x0.device
+        res = dict(x=torch.empty_like(x0), f=torch.empty(B, dtype=torch.float64, device=dev))
+        for k in ("status", "nit", "violation", "best_start"):
+            res[k] = torch.empty(B, dtype=torch.int32, device=dev)
+        res["start_max_violation"] = torch.empty((B, K), dtype=torch.float64, device=dev)
+        if return_all:
+            res["all"] = dict(x=torch.empty((B, K, lay.n), dtype=torch.float64, device=dev),
+                              f=torch.empty((B, K), dtype=torch.float64, device=dev),
+                              **{k: torch.empty((B, K), dtype=torch.int32, device=dev) for k in ("status", "nit", "violation")})
+        outs.append(res)
+        per = max(1, MULTISTART_ROWS // K)
+        pieces += [(j, lo, min(B, lo + per)) for lo in range(0, B, per)]
+    waves, rows = [[]], 0
+    for j, lo, hi in pieces:
+        if waves[-1] and rows + (hi - lo) * K > MULTISTART_ROWS:
+            waves.append([])
+            rows = 0
+        waves[-1].append((j, lo, hi))
+        rows += (hi - lo) * K
+    for wave in waves:
+        if not wave:
+            continue
+        expanded = []
+        for j, lo, hi in wave:
+            spec, par, x0 = buckets[j]
+            expanded.append((spec,) + multistart_expand(spec, par[lo:hi], x0[lo:hi], K, seed, spread))
+        if len(expanded) == 1:
+            sols = [solve(*expanded[0], maxiter=maxiter, ftol=ftol, jacobian=jacobian)]
+        else:
+            sols = solve_mixed(expanded, maxiter, ftol, jacobian)
+        for (j, lo, hi), sol in zip(wave, sols):
+            spec, par, _ = buckets[j]
+            res = outs[j]
+            multistart_select(spec, par[lo:hi], sol, K, tol, out={k: res[k][lo:hi] for k in (
+                "x", "f", "status", "nit", "violation", "best_start", "start_max_violation")})
+            if return_all:
+                for k in ("x", "f", "status", "nit", "violation"):
+                    res["all"][k][lo:hi] = sol[k].view(res["all"][k][lo:hi].shape)
+    for res in outs:
+        mv = res.pop("start_max_violation")
+        res["max_violation"] = mv.gather(1, res["best_start"].long()[:, None])[:, 0]
+        if return_all:
+            res["all"]["max_violation"] = mv
+    return outs
+
+
+def solve_multistart(spec, par, x0, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100, ftol=1e-6,
+                     jacobian="analytic", return_all=False):
+    """Multi-start solve of B problems of one shape (see ``solve_mixed_multistart``).  starts = 1 returns exactly what
+    ``solve`` returns for x0 (start 0 is x0 itself), plus best_start = 0 and max_violation."""
+    return solve_mixed_multistart([(spec, par, x0)], starts, seed, spread, tol, maxiter, ftol, jacobian, return_all)[0]

@@ -855,6 +855,66 @@ extern "C" int tg_solve_mixed_batch(int nbuckets, const int *specs, const int *c
 }
 
 // ---------------------------------------------------------------------------
+// multi-start solves: expansion of B problems into B * K seeded starts (tg_multistart.cu), and the selection of the best
+// start per problem after the caller's ordinary solve of the B * K rows (tg_kernels_eval.inc, planned as tg_eval_batch)
+// ---------------------------------------------------------------------------
+static int tg_multistart_args(const char *what, int B, int K)
+{
+    if (K < 1) return tg_fail(2, (std::string(what) + ": the number of starts K must be at least 1").c_str());
+    if ((long long)B * K > 0x7fffffffLL) return tg_fail(2, (std::string(what) + ": B * K exceeds the int range").c_str());
+    return 0;
+}
+
+extern "C" int tg_multistart_expand(const int *spec, int B, int K, const double *par, const double *x0,
+                                    unsigned long long seed, double spread, double *par_out, double *x_out, void *stream)
+{
+    TgShape S;
+    int rc = tg_make_shape(spec, &S);
+    if (rc || (rc = tg_multistart_args("tg_multistart_expand", B, K))) return rc;
+    if (!(spread >= 0 && spread <= 1e300)) return tg_fail(2, "tg_multistart_expand: spread must be finite and >= 0");
+    if (B <= 0) return 0;
+    if (!par || !x0 || !par_out || !x_out) return tg_fail(1, "tg_multistart_expand: NULL argument");
+    if ((rc = tg_device_check())) return rc;
+    cudaError_t e = tg_launch_multistart_expand(S.L, B, K, par, x0, seed, spread, par_out, x_out, g_sm_count, (cudaStream_t)stream);
+    g_launches++;
+    if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_multistart_expand_kernel launch", e);
+    return 0;
+}
+
+extern "C" int tg_multistart_select(const int *spec, int B, int K, const double *par, const double *xs, const double *f,
+                                    const int *status, const int *nit, const int *violation, double tol, double *x_best,
+                                    double *f_best, int *status_best, int *nit_best, int *violation_best, int *best_start,
+                                    double *max_violation, void *stream)
+{
+    TgShape S;
+    int rc = tg_make_shape(spec, &S);
+    if (rc || (rc = tg_multistart_args("tg_multistart_select", B, K))) return rc;
+    if (B <= 0) return 0;
+    if (!par || !xs || !f || !status || !nit || !violation || !x_best || !f_best || !status_best || !nit_best ||
+        !violation_best || !best_start)
+        return tg_fail(1, "tg_multistart_select: NULL argument (only max_violation may be NULL)");
+    if ((rc = tg_device_check())) return rc;
+    const int gs = tg_env_gs("TG_EVAL_GS", tg_default_gs(S.L));
+    const int groups = tg_eval_groups(S.L, gs, true, g_smem_optin);
+    const size_t need = (size_t)tg_eval_group_doubles(S.L, true) * sizeof(double);
+    if (groups == 0) {
+        snprintf(g_err, sizeof g_err, "tg_select_kernel: a problem with n = %d, m = %d needs %zu bytes of shared memory, "
+                 "more than the device's %d", S.L.n, S.L.m, need, g_smem_optin);
+        return 3;
+    }
+    int grid = (B + groups - 1) / groups;
+    if (grid > g_sm_count * 32) grid = g_sm_count * 32;
+    const TgSelectLaunch a = {S, B, K, par, xs, f, status, nit, violation, tol, x_best, f_best, status_best, nit_best,
+                              violation_best, best_start, max_violation, tg_plan_fix(S), grid, groups, groups * need,
+                              (cudaStream_t)stream};
+    static cudaError_t (*const launchers[3])(const TgSelectLaunch &) = {tg_launch_select_g8, tg_launch_select_g16, tg_launch_select_g32};
+    cudaError_t e = launchers[tg_lanes_index(gs)](a);
+    g_launches++;
+    if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_select_kernel launch", e);
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
 // the reference's 24 symbols: single-problem launches (one warp)
 // ---------------------------------------------------------------------------
 enum { LG_TURN = 0, LG_MINV, LG_OBST, LG_INTERVALS, LG_BEZ };

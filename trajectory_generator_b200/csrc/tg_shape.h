@@ -153,6 +153,28 @@ struct TgEvalLaunch {
 cudaError_t tg_launch_eval_g8(const TgEvalLaunch &a), tg_launch_eval_g16(const TgEvalLaunch &a), tg_launch_eval_g32(const TgEvalLaunch &a);
 cudaError_t tg_launch_linear_g32(const TgShape &S, int B, const double *par, double *alin, int sm_count, cudaStream_t st);
 
+// Multi-start selection kernel (tg_kernels_eval.inc, planned like the evaluation kernel by tg_multistart_select): one
+// lane group per problem, its K starts' rows xs / f / status / nit / violation at b * K + k
+struct TgSelectLaunch {
+    TgShape S;
+    int B, K;
+    const double *par, *xs, *f;
+    const int *status, *nit, *violation;
+    double tol;
+    double *x_best, *f_best;
+    int *status_best, *nit_best, *violation_best, *best_start;
+    double *max_violation;      // [B * K] or nullptr
+    int fix, grid, groups;
+    size_t smem;
+    cudaStream_t st;
+};
+cudaError_t tg_launch_select_g8(const TgSelectLaunch &a), tg_launch_select_g16(const TgSelectLaunch &a),
+    tg_launch_select_g32(const TgSelectLaunch &a);
+// Multi-start expansion (tg_multistart.cu)
+cudaError_t tg_launch_multistart_expand(const TgLayout &L, int B, int K, const double *par, const double *x0,
+                                        unsigned long long seed, double spread, double *par_out, double *x_out,
+                                        int sm_count, cudaStream_t st);
+
 // launch counter of the library (tg_launch_count), for kernels launched outside tg_api.cu
 void tg_note_launch(int count);
 

@@ -17,9 +17,12 @@ from .problem import PackedGroup, pack_problem, pack_problems
 class TrajectoryResult:
     """Per-problem solver outcome that the reference keeps internal (OptimizeResult.status / nit / fun)."""
 
-    def __init__(self, control_points, scale_factor, is_violation, status, nit, fun, x):
+    def __init__(self, control_points, scale_factor, is_violation, status, nit, fun, x, start=0, max_violation=None):
+        """start: the multi-start start that won (0 without multi-start); max_violation: its true maximum constraint
+        violation (computed by multi-start solves only, else None)."""
         self.control_points, self.scale_factor, self.is_violation = control_points, scale_factor, is_violation
         self.status, self.nit, self.fun, self.x = status, nit, fun, x
+        self.start, self.max_violation = start, max_violation
         self.success = status == 0
 
     def __iter__(self):      # unpacks like the reference's return tuple
@@ -27,16 +30,22 @@ class TrajectoryResult:
 
 
 class TrajectoryGenerator:
-    def __init__(self, dimension: int, jacobian: str = "fd", maxiter: int = 100, ftol: float = 1e-6):
+    def __init__(self, dimension: int, jacobian: str = "fd", maxiter: int = 100, ftol: float = 1e-6, starts: int = 1,
+                 seed: int = 0):
         """jacobian: "fd" (default) forms derivatives on the GPU exactly as scipy does for the reference (2-point
         forward differences, h = 1.49e-8, bound-aware), so the iterates follow the reference's and the converged
         control points agree within 1e-5 wherever the reference reproduces itself to that level; "analytic" uses
         the closed-form Jacobians (1.3-1.8x faster; same optimum within what ftol resolves, different last digits).
         maxiter / ftol default to scipy's SLSQP defaults, which is what the reference runs with
-        (TG/trajectory_generator.py:85)."""
+        (TG/trajectory_generator.py:85).
+        starts > 1: every problem is solved from `starts` seeded starts on the device (start 0 is the usual one) and the
+        best converged feasible result is kept (batch.solve_mixed_multistart; DESIGN.md §4 *Multi-start*)."""
+        if int(starts) < 1:
+            raise ValueError("starts must be at least 1")
         self._dimension = dimension
         self._order = 3
         self._jacobian, self._maxiter, self._ftol = jacobian, maxiter, ftol
+        self._starts, self._seed = int(starts), int(seed)
         self.last_result = None
 
     # ---- reference API ---------------------------------------------------------------------------
@@ -107,6 +116,8 @@ class TrajectoryGenerator:
 
     def _solve_groups(self, groups, results, offset):
         """one library call for the groups (shapes) of a chunk; results[offset + index] are filled in"""
+        if self._starts > 1:
+            return self._solve_groups_multistart(groups, results, offset)
         buckets = [(g.spec, g.par, g.x0) for g in groups]
         if len(buckets) == 1:
             outs = [batch.solve_host(*buckets[0], self._maxiter, self._ftol, self._jacobian)]
@@ -120,4 +131,23 @@ class TrajectoryGenerator:
             nit = out["nit"].tolist(); fs = out["f"].tolist()
             for k, i in enumerate(idx.tolist()):
                 results[offset + i] = TrajectoryResult(cps_all[k], scales[k], bool(viol[k]), status[k], nit[k], fs[k], xs[k])
+        return results
+
+    def _solve_groups_multistart(self, groups, results, offset):
+        """the groups moved to the current CUDA device and solved from self._starts starts each"""
+        import torch
+        dev = torch.device("cuda", torch.cuda.current_device())
+        buckets = [(g.spec, torch.from_numpy(np.ascontiguousarray(g.par)).to(dev),
+                    torch.from_numpy(np.ascontiguousarray(g.x0)).to(dev)) for g in groups]
+        outs = batch.solve_mixed_multistart(buckets, self._starts, self._seed, maxiter=self._maxiter, ftol=self._ftol,
+                                            jacobian=self._jacobian)
+        for g, out in zip(groups, outs):
+            lay, idx = g.layout, g.indices
+            out = {k: v.cpu().numpy() for k, v in out.items()}
+            xs = out["x"]
+            cps_all = xs[:, :lay.d * lay.N].reshape(len(idx), lay.d, lay.N).copy()
+            for k, i in enumerate(idx.tolist()):
+                results[offset + i] = TrajectoryResult(cps_all[k], float(xs[k, lay.ia]), bool(out["violation"][k]),
+                                                       int(out["status"][k]), int(out["nit"][k]), float(out["f"][k]), xs[k],
+                                                       int(out["best_start"][k]), float(out["max_violation"][k]))
         return results
