@@ -84,6 +84,22 @@ int tg_solve_plan_info(const int *spec, int B, int *out, int cap);
 int tg_solve_batch(const int *spec, int B, const double *par, double *x, double *f,
                    int *status, int *nit, int *violation, int maxiter, double ftol, int flags,
                    void *workspace, size_t workspace_bytes, void *stream);
+/*
+ * tg_solve_batch plus, unless NULL, per problem:
+ *   lam[B*m]  the KKT multipliers of the last QP in constraint row order (scipy's OptimizeResult.multipliers: the
+ *             equality rows, then the inequality rows; no bound multipliers).  The terminal location rows, which the
+ *             QP eliminates, get theirs from the QP's stationarity on the eliminated coordinates (csrc/tg_sqp.h,
+ *             tg_sqp_kkt).  For status != 0 they are the last successful QP's values.
+ *   kkt[B*4]  first-order optimality certificate at the returned x, absolute, NaN = +inf, with the derivatives the
+ *             solve used (analytic or finite-difference) and gradL = g - sum_j lam_j grad c_j:
+ *             [0] stationarity max_i |gradL_i| (only its infeasible sign at a variable on its bound),
+ *             [1] infeasibility max |c_j| (equality rows), max(0, -c_j) (inequality rows),
+ *             [2] dual infeasibility max(0, -lam_j), [3] complementarity max |lam_j c_j| (inequality rows).
+ * x, f, status, nit and violation are those of tg_solve_batch.
+ */
+int tg_solve_batch_kkt(const int *spec, int B, const double *par, double *x, double *f,
+                       int *status, int *nit, int *violation, int maxiter, double ftol, int flags,
+                       void *workspace, size_t workspace_bytes, void *stream, double *lam, double *kkt);
 
 /* host-buffer variants: copy in, launch, copy out (the reference-facing call measured as `e2e`) */
 int tg_eval_host(const int *spec, int B, const double *par, const double *x,
@@ -108,6 +124,12 @@ int tg_solve_mixed_host(int nbuckets, const int *specs, const int *counts, const
 int tg_solve_mixed_batch(int nbuckets, const int *specs, const int *counts, const double *const *par, double *const *x,
                          double *const *f, int *const *status, int *const *nit, int *const *violation, int maxiter,
                          double ftol, int flags, void *stream);
+/* the same with tg_solve_batch_kkt's outputs: lam[k] (counts[k] * m of bucket k) and kkt[k] (counts[k] * 4) are device
+ * buffers; lam, kkt or any entry of them may be NULL */
+int tg_solve_mixed_batch_kkt(int nbuckets, const int *specs, const int *counts, const double *const *par,
+                             double *const *x, double *const *f, int *const *status, int *const *nit,
+                             int *const *violation, int maxiter, double ftol, int flags, void *stream,
+                             double *const *lam, double *const *kkt);
 
 /*
  * Multi-start solves: K seeded starts per problem, solved as ordinary problems, the best one kept.  The problems are

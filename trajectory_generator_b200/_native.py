@@ -98,6 +98,7 @@ def lib():
         L.tg_solve_plan_info.restype = ctypes.c_int
         L.tg_solve_batch.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_double,
                                      ctypes.c_int, vp, sz, vp]
+        L.tg_solve_batch_kkt.argtypes = list(L.tg_solve_batch.argtypes) + [vp, vp]
         L.tg_eval_host.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp, vp]
         L.tg_solve_host.argtypes = [_I32, ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_double,
                                     ctypes.c_int]
@@ -132,7 +133,7 @@ def lib():
         L.tg_multistart_expand.restype = ctypes.c_int
         L.tg_multistart_select.argtypes = [_I32, ctypes.c_int, ctypes.c_int] + [vp] * 6 + [ctypes.c_double] + [vp] * 8
         L.tg_multistart_select.restype = ctypes.c_int
-        for name in ("tg_eval_batch", "tg_linear_rows_batch", "tg_solve_batch", "tg_eval_host", "tg_solve_host"):
+        for name in ("tg_eval_batch", "tg_linear_rows_batch", "tg_solve_batch", "tg_solve_batch_kkt", "tg_eval_host", "tg_solve_host"):
             getattr(L, name).restype = ctypes.c_int
         _LIB = L
     return _LIB

@@ -8,6 +8,10 @@ host-buffer (numpy, copies inside the C call) variants of
   * ``solve``     -- M2: the scipy SLSQP call of TG/trajectory_generator.py:87-94 for B problems;
   * ``solve_multistart`` -- M2 from K seeded starts per problem, the best converged feasible result kept (opt-in).
 
+Every solve entry point takes ``multipliers=False``; with True its result also holds ``lam`` [B, m], the KKT
+multipliers of the last QP in constraint row order (scipy's ``OptimizeResult.multipliers``; ``Layout.row_blocks`` names
+the rows), and ``kkt`` [B, 4], the first-order optimality certificate at the returned x (KKT_FIELDS; DESIGN.md §4).
+
 PyTorch is used only to own device memory and streams.
 """
 import ctypes
@@ -18,6 +22,8 @@ from . import _native
 from .problem import Layout
 
 JACOBIAN_MODES = {"analytic": 0, "fd": 1}     # "fd": scipy's forward differences emulated on the GPU
+# entries of `kkt` (include/trajectory_generator_b200.h, tg_solve_batch_kkt): absolute, NaN = +inf
+KKT_FIELDS = ("stationarity", "infeasibility", "dual_infeasibility", "complementarity")
 
 
 def _torch():
@@ -108,9 +114,15 @@ def _flags(jacobian, fused):
     return JACOBIAN_MODES[jacobian] | (2 if fused else 0)
 
 
-def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=None, fused=False):
+def _kkt_outputs(torch, lay, B, dev):
+    return dict(lam=torch.empty((B, lay.m), dtype=torch.float64, device=dev),
+                kkt=torch.empty((B, 4), dtype=torch.float64, device=dev))
+
+
+def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=None, fused=False, multipliers=False):
     """Device-resident M2 solve.  x [B,n] is overwritten with the optimised variables.
-    Returns dict(x, f, status, nit, violation) of CUDA tensors.
+    Returns dict(x, f, status, nit, violation) of CUDA tensors; with multipliers=True also lam [B, m] and kkt [B, 4]
+    (tg_solve_batch_kkt), new tensors of every call.
     fused=False (default): lock-step stage kernels over the whole batch; fused=True: one persistent kernel in
     which each warp runs a whole solve (same arithmetic, kept for comparison)."""
     torch = _torch()
@@ -128,12 +140,16 @@ def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=Non
     buf = buffers if buffers is not None else SolveBuffers(spec, B, dev)
     if buf.B < B or not np.array_equal(buf.spec, np.ascontiguousarray(spec, dtype=np.int32)) or buf.ws.device != dev:
         raise ValueError("the SolveBuffers were made for another shape, a smaller batch or another device")
+    args = (buf.sp, B, _ptr(par), _ptr(x), _ptr(buf.f), _ptr(buf.status), _ptr(buf.nit), _ptr(buf.violation),
+            int(maxiter), float(ftol), _flags(jacobian, fused), _ptr(buf.ws), buf.ws.numel(), _stream(torch, dev))
+    extra = _kkt_outputs(torch, lay, B, dev) if multipliers else {}
     with torch.cuda.device(dev):
-        rc = _native.lib().tg_solve_batch(buf.sp, B, _ptr(par), _ptr(x), _ptr(buf.f), _ptr(buf.status), _ptr(buf.nit),
-                                          _ptr(buf.violation), int(maxiter), float(ftol), _flags(jacobian, fused),
-                                          _ptr(buf.ws), buf.ws.numel(), _stream(torch, dev))
-    _native.check(rc, "tg_solve_batch")
-    return dict(x=x, f=buf.f, status=buf.status, nit=buf.nit, violation=buf.violation)
+        if multipliers:
+            rc = _native.lib().tg_solve_batch_kkt(*args, _ptr(extra["lam"]), _ptr(extra["kkt"]))
+        else:
+            rc = _native.lib().tg_solve_batch(*args)
+    _native.check(rc, "tg_solve_batch_kkt" if multipliers else "tg_solve_batch")
+    return dict(x=x, f=buf.f, status=buf.status, nit=buf.nit, violation=buf.violation, **extra)
 
 
 def _np_ptr(a):
@@ -226,11 +242,12 @@ def solve_mixed_host(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
     return outs
 
 
-def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
+def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic", multipliers=False):
     """Device-resident M2 solve of problems of DIFFERENT shapes in one call (tg_solve_mixed_batch).
     buckets: list of (spec, par [Bk, P], x [Bk, n]) CUDA tensors; x is overwritten with the solution.  The buckets run
     concurrently on internal streams that fork from and join the current stream.  Returns one dict(x, f, status, nit,
-    violation) of CUDA tensors per bucket."""
+    violation) of CUDA tensors per bucket; with multipliers=True each also holds lam [Bk, m] and kkt [Bk, 4]
+    (tg_solve_mixed_batch_kkt)."""
     torch = _torch()
     L = _native.lib()
     nb = len(buckets)
@@ -240,7 +257,7 @@ def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
     specs = np.zeros((nb, nspec), dtype=np.int32)
     counts = np.zeros(nb, dtype=np.int32)
     vp_array = ctypes.c_void_p * nb
-    ptrs = {k: vp_array() for k in ("par", "x", "f", "status", "nit", "violation")}
+    ptrs = {k: vp_array() for k in ("par", "x", "f", "status", "nit", "violation", "lam", "kkt")}
     outs, keep = [], []
     dev = buckets[0][2].device
     for k, (spec, par, x) in enumerate(buckets):
@@ -256,18 +273,22 @@ def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
         counts[k] = B
         out = dict(x=x, f=torch.empty(B, dtype=torch.float64, device=dev), status=torch.empty(B, dtype=torch.int32, device=dev),
                    nit=torch.empty(B, dtype=torch.int32, device=dev), violation=torch.empty(B, dtype=torch.int32, device=dev))
+        if multipliers:
+            out.update(_kkt_outputs(torch, lay, B, dev))
         outs.append(out); keep.append(par)
         ptrs["par"][k] = par.data_ptr()
-        for name in ("x", "f", "status", "nit", "violation"):
+        for name in ("x", "f", "status", "nit", "violation") + (("lam", "kkt") if multipliers else ()):
             ptrs[name][k] = out[name].data_ptr()
-    L.tg_solve_mixed_batch.restype = ctypes.c_int
-    L.tg_solve_mixed_batch.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_void_p] * 6 + \
-                                      [ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_void_p]
+    args = (nb, specs.ctypes.data, counts.ctypes.data, ptrs["par"], ptrs["x"], ptrs["f"], ptrs["status"], ptrs["nit"],
+            ptrs["violation"], int(maxiter), float(ftol), _flags(jacobian, False), _stream(torch, dev))
+    name = "tg_solve_mixed_batch_kkt" if multipliers else "tg_solve_mixed_batch"
+    fn = getattr(L, name)
+    fn.restype = ctypes.c_int
+    fn.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_void_p] * 6 + \
+        [ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_void_p] + [ctypes.c_void_p] * (2 if multipliers else 0)
     with torch.cuda.device(dev):
-        rc = L.tg_solve_mixed_batch(nb, specs.ctypes.data, counts.ctypes.data, ptrs["par"], ptrs["x"], ptrs["f"], ptrs["status"],
-                                    ptrs["nit"], ptrs["violation"], int(maxiter), float(ftol), _flags(jacobian, False),
-                                    _stream(torch, dev))
-    _native.check(rc, "tg_solve_mixed_batch")
+        rc = fn(*args, ptrs["lam"], ptrs["kkt"]) if multipliers else fn(*args)
+    _native.check(rc, name)
     return outs
 
 
@@ -345,13 +366,14 @@ def multistart_select(spec, par, sol, starts, tol=MULTISTART_TOL, out=None):
 
 
 def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100,
-                           ftol=1e-6, jacobian="analytic", return_all=False):
+                           ftol=1e-6, jacobian="analytic", return_all=False, multipliers=False):
     """Multi-start solve of problems of one or several shapes: buckets = list of (spec, par [Bk, P], x0 [Bk, n]) CUDA
     tensors (x0 is not modified).  Per bucket: expand -> solve -> select on the current stream, in pieces of at most
     MULTISTART_ROWS expanded rows; the pieces of several shapes go through one ``solve_mixed`` call.  Returns one dict
     per bucket: the B-row dict of ``solve`` plus best_start and max_violation (the winner's true maximum violation);
     with return_all, also "all": the K per-start results, dict(x [B, K, n], f, status, nit, violation,
-    max_violation [B, K])."""
+    max_violation [B, K]).  multipliers=True adds the winner's lam [B, m] and kkt [B, 4] (and every start's,
+    [B, K, m] and [B, K, 4], under "all")."""
     torch = _torch()
     K = int(starts)
     if K < 1:
@@ -364,10 +386,15 @@ def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, to
         for k in ("status", "nit", "violation", "best_start"):
             res[k] = torch.empty(B, dtype=torch.int32, device=dev)
         res["start_max_violation"] = torch.empty((B, K), dtype=torch.float64, device=dev)
+        if multipliers:
+            res.update(_kkt_outputs(torch, lay, B, dev))
         if return_all:
             res["all"] = dict(x=torch.empty((B, K, lay.n), dtype=torch.float64, device=dev),
                               f=torch.empty((B, K), dtype=torch.float64, device=dev),
                               **{k: torch.empty((B, K), dtype=torch.int32, device=dev) for k in ("status", "nit", "violation")})
+            if multipliers:
+                res["all"].update(lam=torch.empty((B, K, lay.m), dtype=torch.float64, device=dev),
+                                  kkt=torch.empty((B, K, 4), dtype=torch.float64, device=dev))
         outs.append(res)
         per = max(1, MULTISTART_ROWS // K)
         pieces += [(j, lo, min(B, lo + per)) for lo in range(0, B, per)]
@@ -386,16 +413,20 @@ def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, to
             spec, par, x0 = buckets[j]
             expanded.append((spec,) + multistart_expand(spec, par[lo:hi], x0[lo:hi], K, seed, spread))
         if len(expanded) == 1:
-            sols = [solve(*expanded[0], maxiter=maxiter, ftol=ftol, jacobian=jacobian)]
+            sols = [solve(*expanded[0], maxiter=maxiter, ftol=ftol, jacobian=jacobian, multipliers=multipliers)]
         else:
-            sols = solve_mixed(expanded, maxiter, ftol, jacobian)
+            sols = solve_mixed(expanded, maxiter, ftol, jacobian, multipliers)
         for (j, lo, hi), sol in zip(wave, sols):
             spec, par, _ = buckets[j]
             res = outs[j]
             multistart_select(spec, par[lo:hi], sol, K, tol, out={k: res[k][lo:hi] for k in (
                 "x", "f", "status", "nit", "violation", "best_start", "start_max_violation")})
+            if multipliers:
+                rows = torch.arange(hi - lo, device=par.device) * K + res["best_start"][lo:hi].long()
+                res["lam"][lo:hi] = sol["lam"][rows]
+                res["kkt"][lo:hi] = sol["kkt"][rows]
             if return_all:
-                for k in ("x", "f", "status", "nit", "violation"):
+                for k in ("x", "f", "status", "nit", "violation") + (("lam", "kkt") if multipliers else ()):
                     res["all"][k][lo:hi] = sol[k].view(res["all"][k][lo:hi].shape)
     for res in outs:
         mv = res.pop("start_max_violation")
@@ -406,7 +437,8 @@ def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, to
 
 
 def solve_multistart(spec, par, x0, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100, ftol=1e-6,
-                     jacobian="analytic", return_all=False):
+                     jacobian="analytic", return_all=False, multipliers=False):
     """Multi-start solve of B problems of one shape (see ``solve_mixed_multistart``).  starts = 1 returns exactly what
     ``solve`` returns for x0 (start 0 is x0 itself), plus best_start = 0 and max_violation."""
-    return solve_mixed_multistart([(spec, par, x0)], starts, seed, spread, tol, maxiter, ftol, jacobian, return_all)[0]
+    return solve_mixed_multistart([(spec, par, x0)], starts, seed, spread, tol, maxiter, ftol, jacobian, return_all,
+                                  multipliers)[0]

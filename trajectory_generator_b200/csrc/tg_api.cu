@@ -388,8 +388,8 @@ static cudaError_t tg_launch_stage(const TgStageLauncher launchers[4], const TgS
 }
 
 static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const double *par, double *x, double *f,
-                           int *status, int *nit, int *violation, int maxiter, double ftol, int flags, void *workspace,
-                           cudaStream_t st)
+                           int *status, int *nit, int *violation, double *lam, double *kkt, int maxiter, double ftol,
+                           int flags, void *workspace, cudaStream_t st)
 {
     const TgLayout &L = S.L;
     char *wsb = (char *)workspace;
@@ -463,7 +463,8 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
             Slice &q = sl[k];
             const int o = lo + q.lo;
             TG_LAUNCH(tg_launch_finish_g32(S, q.nb, q.pws, P.np, x + (size_t)o * L.n, f ? f + o : nullptr, status ? status + o : nullptr,
-                                           nit ? nit + o : nullptr, violation ? violation + o : nullptr, q.rc, q.st),
+                                           nit ? nit + o : nullptr, violation ? violation + o : nullptr,
+                                           lam ? lam + (size_t)o * L.m : nullptr, kkt ? kkt + (size_t)o * 4 : nullptr, q.rc, q.st),
                       "tg_sqp_finish_kernel");
             if (ns > 1) {
                 TG_CUDA(cudaEventRecord(ss->join[k], q.st));
@@ -491,9 +492,9 @@ static int tg_solve_phased(const TgShape &S, const TgSolvePlan &P, int B, const 
     return 0;
 }
 
-extern "C" int tg_solve_batch(const int *spec, int B, const double *par, double *x, double *f, int *status, int *nit,
-                              int *violation, int maxiter, double ftol, int flags, void *workspace,
-                              size_t workspace_bytes, void *stream)
+extern "C" int tg_solve_batch_kkt(const int *spec, int B, const double *par, double *x, double *f, int *status, int *nit,
+                                  int *violation, int maxiter, double ftol, int flags, void *workspace,
+                                  size_t workspace_bytes, void *stream, double *lam, double *kkt)
 {
     TgShape S;
     TgSolvePlan P;
@@ -506,11 +507,19 @@ extern "C" int tg_solve_batch(const int *spec, int B, const double *par, double 
     if (flags & TG_SOLVE_FUSED) {
         int *counters = (int *)workspace;
         TG_CUDA(cudaMemsetAsync(counters, 0, 256, st));
-        TG_LAUNCH(tg_launch_fused_g32(S, B, par, x, f, status, nit, violation, maxiter, ftol, flags, (char *)workspace + 256,
+        TG_LAUNCH(tg_launch_fused_g32(S, B, par, x, f, status, nit, violation, lam, kkt, maxiter, ftol, flags, (char *)workspace + 256,
                                       counters, g_sm_count, g_smem_optin, st), "tg_solve_kernel");
         return 0;
     }
-    return tg_solve_phased(S, P, B, par, x, f, status, nit, violation, maxiter, ftol, flags, workspace, st);
+    return tg_solve_phased(S, P, B, par, x, f, status, nit, violation, lam, kkt, maxiter, ftol, flags, workspace, st);
+}
+
+extern "C" int tg_solve_batch(const int *spec, int B, const double *par, double *x, double *f, int *status, int *nit,
+                              int *violation, int maxiter, double ftol, int flags, void *workspace,
+                              size_t workspace_bytes, void *stream)
+{
+    return tg_solve_batch_kkt(spec, B, par, x, f, status, nit, violation, maxiter, ftol, flags, workspace, workspace_bytes,
+                              stream, nullptr, nullptr);
 }
 
 // ---------------------------------------------------------------------------
@@ -716,7 +725,8 @@ static TgMixedCtx g_mixed_ctx[TG_MAX_DEVICES];
 // pointers: the buckets' streams fork from and join the caller's stream)
 static int tg_solve_mixed_impl(bool host, int nbuckets, const int *specs, const int *counts, const double *const *par,
                                double *const *x, double *const *f, int *const *status, int *const *nit,
-                               int *const *violation, int maxiter, double ftol, int flags, cudaStream_t caller)
+                               int *const *violation, double *const *lam, double *const *kkt, int maxiter, double ftol,
+                               int flags, cudaStream_t caller)
 {
     if (nbuckets <= 0) return 0;
     if (!specs || !counts || !par || !x) return tg_fail(1, "tg_solve_mixed: NULL argument");
@@ -812,8 +822,9 @@ static int tg_solve_mixed_impl(bool host, int nbuckets, const int *specs, const 
                 if (nit && nit[k]) cp(nit[k], di + B, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost);
                 if (violation && violation[k]) cp(violation[k], di + 2 * B, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost);
             } else if (!r) {
-                r = tg_solve_batch(spec, B, par[k], x[k], f ? f[k] : nullptr, status ? status[k] : nullptr, nit ? nit[k] : nullptr,
-                                   violation ? violation[k] : nullptr, maxiter, ftol, flags, s.ws.p, wsb, s.st);
+                r = tg_solve_batch_kkt(spec, B, par[k], x[k], f ? f[k] : nullptr, status ? status[k] : nullptr,
+                                       nit ? nit[k] : nullptr, violation ? violation[k] : nullptr, maxiter, ftol, flags, s.ws.p,
+                                       wsb, s.st, lam ? lam[k] : nullptr, kkt ? kkt[k] : nullptr);
             }
             // (the slot's workspace and staging buffers are reused by this worker's next bucket, which is queued on the
             // same stream; host buffers must be complete before the call returns)
@@ -843,15 +854,25 @@ extern "C" int tg_solve_mixed_host(int nbuckets, const int *specs, const int *co
                                    double *const *x, double *const *f, int *const *status, int *const *nit,
                                    int *const *violation, int maxiter, double ftol, int flags)
 {
-    return tg_solve_mixed_impl(true, nbuckets, specs, counts, par, x, f, status, nit, violation, maxiter, ftol, flags, nullptr);
+    return tg_solve_mixed_impl(true, nbuckets, specs, counts, par, x, f, status, nit, violation, nullptr, nullptr, maxiter, ftol,
+                               flags, nullptr);
+}
+
+extern "C" int tg_solve_mixed_batch_kkt(int nbuckets, const int *specs, const int *counts, const double *const *par,
+                                        double *const *x, double *const *f, int *const *status, int *const *nit,
+                                        int *const *violation, int maxiter, double ftol, int flags, void *stream,
+                                        double *const *lam, double *const *kkt)
+{
+    return tg_solve_mixed_impl(false, nbuckets, specs, counts, par, x, f, status, nit, violation, lam, kkt, maxiter, ftol, flags,
+                               (cudaStream_t)stream);
 }
 
 extern "C" int tg_solve_mixed_batch(int nbuckets, const int *specs, const int *counts, const double *const *par,
                                     double *const *x, double *const *f, int *const *status, int *const *nit,
                                     int *const *violation, int maxiter, double ftol, int flags, void *stream)
 {
-    return tg_solve_mixed_impl(false, nbuckets, specs, counts, par, x, f, status, nit, violation, maxiter, ftol, flags,
-                               (cudaStream_t)stream);
+    return tg_solve_mixed_batch_kkt(nbuckets, specs, counts, par, x, f, status, nit, violation, maxiter, ftol, flags, stream,
+                                    nullptr, nullptr);
 }
 
 // ---------------------------------------------------------------------------

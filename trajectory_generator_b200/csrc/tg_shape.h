@@ -134,11 +134,11 @@ struct TgStageLaunch {
 cudaError_t tg_launch_ls_g8(const TgStageLaunch &a), tg_launch_ls_g16(const TgStageLaunch &a), tg_launch_ls_g32(const TgStageLaunch &a);
 cudaError_t tg_launch_fd_g8(const TgStageLaunch &a), tg_launch_fd_g16(const TgStageLaunch &a), tg_launch_fd_g32(const TgStageLaunch &a);
 cudaError_t tg_launch_qp_g16(const TgStageLaunch &a), tg_launch_qp_g32(const TgStageLaunch &a), tg_launch_qp_g64(const TgStageLaunch &a);
-// once per solve (32 lanes)
+// once per solve (32 lanes); the finish kernel writes lam[B*m] / kkt[B*4] (tg_sqp_kkt) unless they are null
 cudaError_t tg_launch_begin_g32(const TgShape &S, int B, const double *x, double *pws, size_t np, int maxiter, double ftol,
                                 int flags, TgRoundCtl *rc, int *list0, cudaStream_t st);
 cudaError_t tg_launch_finish_g32(const TgShape &S, int B, const double *pws, size_t np, double *x, double *f, int *status,
-                                 int *nit, int *violation, TgRoundCtl *rc, cudaStream_t st);
+                                 int *nit, int *violation, double *lam, double *kkt, TgRoundCtl *rc, cudaStream_t st);
 
 // Evaluation kernel (tg_kernels_eval.inc): `groups` lane groups per CTA with `smem` bytes of shared memory
 struct TgEvalLaunch {
@@ -181,6 +181,6 @@ void tg_note_launch(int count);
 // fused kernel (tg_solve_fused.cu, 32 lanes): it sizes its grid and its global workspace itself (the same numbers for both)
 size_t tg_fused_workspace_bytes(const TgShape &S, int B, int sm_count, int smem_optin);
 cudaError_t tg_launch_fused_g32(const TgShape &S, int B, const double *par, double *x, double *f, int *status, int *nit,
-                                int *violation, int maxiter, double ftol, int flags, void *gws, int *queue, int sm_count,
-                                int smem_optin, cudaStream_t st);
+                                int *violation, double *lam, double *kkt, int maxiter, double ftol, int flags, void *gws,
+                                int *queue, int sm_count, int smem_optin, cudaStream_t st);
 #endif

@@ -13,8 +13,9 @@
 template <int D>
 __global__ void __launch_bounds__(128, 4)
 tg_solve_kernel(const TgShape S, int B, const double *__restrict__ par, double *__restrict__ x, double *__restrict__ fout,
-                int *__restrict__ status, int *__restrict__ nit, int *__restrict__ violation, int maxiter, double ftol,
-                int flags, double *gws, size_t ws_doubles, int warps_per_cta, int *queue)
+                int *__restrict__ status, int *__restrict__ nit, int *__restrict__ violation, double *__restrict__ lam,
+                double *__restrict__ kkt, int maxiter, double ftol, int flags, double *gws, size_t ws_doubles,
+                int warps_per_cta, int *queue)
 {
     extern __shared__ double smem[];
     const TgLayout &L = S.L;
@@ -33,11 +34,11 @@ tg_solve_kernel(const TgShape S, int B, const double *__restrict__ par, double *
         tg_sqp_solve<D>(L, S.sp, spar, x + (size_t)b * L.n, ws, maxiter, ftol, flags, &res, nullptr, 0);
         res.status = __shfl_sync(0xffffffffu, res.status, 0);
         int viol = 0;
-        if (res.status != 0) {
-            TgSqpWs W;
-            tg_sqp_carve(L, ws, &W);
-            viol = tg_last_block_violation(L, W.c);
-        }
+        TgSqpWs W;
+        tg_sqp_carve(L, ws, &W);
+        if (res.status != 0) viol = tg_last_block_violation(L, W.c);
+        // (the solve's scratch is free now: its vector u, n + 1 doubles, serves tg_sqp_kkt)
+        if (lam || kkt) tg_sqp_kkt(L, W, lam ? lam + (size_t)b * L.m : nullptr, kkt ? kkt + (size_t)b * 4 : nullptr, W.u);
         if (lane == 0) {
             if (status) status[b] = res.status;
             if (nit) nit[b] = res.nit;
@@ -89,19 +90,19 @@ size_t tg_fused_workspace_bytes(const TgShape &S, int B, int sm_count, int smem_
 }
 
 cudaError_t tg_launch_fused_g32(const TgShape &S, int B, const double *par, double *x, double *f, int *status, int *nit,
-                                int *violation, int maxiter, double ftol, int flags, void *gws, int *queue, int sm_count,
-                                int smem_optin, cudaStream_t st)
+                                int *violation, double *lam, double *kkt, int maxiter, double ftol, int flags, void *gws,
+                                int *queue, int sm_count, int smem_optin, cudaStream_t st)
 {
     const TgFusedPlan P = tg_fused_plan(S, B, sm_count, smem_optin);
     double *ws = P.use_global ? (double *)gws : nullptr;
     cudaError_t e;
     if (S.L.d == 2) {
         if ((e = tg_allow_shared_memory(tg_solve_kernel<2>))) return e;
-        tg_solve_kernel<2><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, maxiter,
+        tg_solve_kernel<2><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, lam, kkt, maxiter,
                                                                                 ftol, flags, ws, P.ws_doubles, P.warps_per_cta, queue);
     } else {
         if ((e = tg_allow_shared_memory(tg_solve_kernel<3>))) return e;
-        tg_solve_kernel<3><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, maxiter,
+        tg_solve_kernel<3><<<P.ctas, P.warps_per_cta * 32, P.smem_bytes, st>>>(S, B, par, x, f, status, nit, violation, lam, kkt, maxiter,
                                                                                 ftol, flags, ws, P.ws_doubles, P.warps_per_cta, queue);
     }
     return cudaGetLastError();

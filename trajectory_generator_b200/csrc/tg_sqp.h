@@ -1744,5 +1744,105 @@ TG_HD int tg_last_block_violation(const TgLayout &L, const double *c)
     return tg_any(bad);
 }
 
+// ---------------------------------------------------------------------------
+// Multipliers and first-order optimality certificate of a finished solve (finish kernel, fused kernel, host build).
+// lam[m]: the multipliers of the last QP in row order -- scipy's OptimizeResult.multipliers (mult[:meq] equality rows,
+// then the inequality rows; no bound multipliers).  The rows the QP eliminates (tg_sqp_pinned) carry a multiplier only
+// while their coordinates still move (tg_qp_solve leaves 0 otherwise); theirs is recovered here from the QP's
+// stationarity on the eliminated coordinates, with gl (the Lagrangian gradient the QP stage formed with the last QP's
+// multipliers), the bound multipliers and the factor L D L' the QP ran with (see below).  Once the pins hold
+// (TgSqpCtl::pins_hold) the factor's pinned rows are frozen, B_Pf is not scipy's, and the recovered multipliers deviate
+// by what DESIGN.md records.  For status != 0 lam is the last successful QP's values with the same recovery (exit 9:
+// the factor may have been updated after that QP; exits 4 / 6: r is zero); they are not checked against an oracle.
+// kkt[4], absolute, NaN -> +inf, with the solver's own derivatives (g, A: analytic or finite-difference, whichever the
+// solve ran) at the returned x and gradL = g - sum_j lam_j grad c_j over the rows with lam_j != 0:
+//   [0] stationarity  max_i |pi_i|, pi_i = min(gradL_i, 0) at x_i == xl_i, max(gradL_i, 0) at x_i == xu_i, else gradL_i
+//   [1] infeasibility max |c_j| (equality rows), max(0, -c_j) (inequality rows)
+//   [2] dual infeasibility max(0, -lam_j) over the inequality rows
+//   [3] complementarity max |lam_j c_j| over the inequality rows
+// Either output may be null.  scratch: tg_sqp_kkt_scratch_doubles(L) doubles (none without eliminated rows).  Every sum
+// runs in a fixed order: the results do not depend on the lanes per problem.
+// ---------------------------------------------------------------------------
+TG_HD size_t tg_sqp_kkt_scratch_doubles(const TgLayout &L) { return tg_sqp_pinned(L) ? (size_t)L.n + (L.n & 1) : 0; }
+
+TG_HD double tg_kkt_fold(double acc, double v) { return v != v ? INFINITY : fmax(acc, v); }
+
+TG_FN void tg_sqp_kkt(const TgLayout &L, const TgSqpWs &W, double *lam, double *kkt, double *scratch)
+{
+    const int lane = TG_LANE(), n = L.n, m = L.m, meq = L.meq;
+    // ---- multipliers of the eliminated rows.  The QP's stationarity in QP order, with d_P = 0 (pins that do not move):
+    // B_ff d_f = -v_f and sigma lambda_P = (B d)_P + v_P, v = gl - (bound multipliers) in rotated space.  With
+    // B = L D L' (free block leading), B_Pf B_ff^-1 = L_Pf L_ff^-1, so sigma lambda_P = v_P - L_Pf L_ff^-1 v_f: one forward
+    // substitution with the free block of the factor, run on into the eliminated rows.  (The stored step s cannot stand
+    // in for d: the line search has scaled it by the product of its trial steps.)  Once the pins hold, L_Pf is frozen
+    // and the term is dropped: sigma lambda_P = v_P agrees better with the full-space subproblem then (DESIGN.md).
+    double *v = W.ne ? scratch : nullptr;
+    if (W.ne) {
+        #pragma unroll 1
+        for (int i = lane; i < n; i += TG_NL) v[tg_qp_index(W, i)] = tg_rot_get(W, W.gl, i) - (W.r[m + i] - W.r[m + W.n1 + i]);
+        TG_SYNC();
+        if (!W.ctl->pins_hold && TG_SERIAL_ACTIVE()) {
+            #pragma unroll 1
+            for (int j = 0; j < W.nf; j++) {
+                const double yj = v[j];
+                #pragma unroll 1
+                for (int k = j + 1 + lane; k < n; k += TG_SERIAL_LANES) v[k] -= W.Lm[j * n + k] * yj;
+                TG_SERIAL_SYNC();
+            }
+        }
+        TG_SYNC();
+        #pragma unroll 1
+        for (int e = lane; e < W.ne; e += TG_NL) {
+            const double rq = W.r[tg_pin_row(W, e)];          // pins that moved in the last QP: the QP formed it
+            v[W.nf + e] = rq != 0 ? rq : v[W.nf + e] / tg_pin_sigma(W, e);
+        }
+        TG_SYNC();
+    }
+    if (lam) {
+        #pragma unroll 1
+        for (int j = lane; j < m; j += TG_NL) lam[j] = W.r[j];
+        TG_SYNC();
+        #pragma unroll 1
+        for (int e = lane; e < W.ne; e += TG_NL) lam[tg_pin_row(W, e)] = v[W.nf + e];
+        TG_SYNC();
+    }
+    if (!kkt) return;
+    // ---- stationarity: the rows of the last QP's active set (W.ract; the only rows with r != 0) and the eliminated rows
+    double st = 0;
+    const int nract = W.ctl->nract;
+    #pragma unroll 1
+    for (int i = lane; i < n; i += TG_NL) {
+        double h = W.g[i];
+        #pragma unroll 1
+        for (int k = 0; k < nract; k++) {
+            const int j = W.ract[k];
+            const double rj = W.r[j];
+            if (rj != 0) h -= (tg_is_sfc_row(W, j) ? tg_sfc_entry(W, W.rot, j, i) : W.A[i * W.lda + tg_arow(W, j)]) * rj;
+        }
+        #pragma unroll 1
+        for (int e = 0; e < W.ne; e++) {
+            const double le = v[W.nf + e];
+            if (le != 0) h -= W.A[i * W.lda + tg_arow(W, tg_pin_row(W, e))] * le;
+        }
+        const double pi = W.x[i] == W.xl[i] ? fmin(h, 0.0) : W.x[i] == W.xu[i] ? fmax(h, 0.0) : h;
+        st = tg_kkt_fold(st, fabs(pi));
+    }
+    // ---- the row folds (the eliminated rows are equality rows: lam_j = r_j over the inequality rows)
+    double inf = 0, dinf = 0, comp = 0;
+    #pragma unroll 1
+    for (int j = lane; j < m; j += TG_NL) {
+        const double cj = W.c[j];
+        if (j < meq) { inf = tg_kkt_fold(inf, fabs(cj)); continue; }
+        const double rj = W.r[j];
+        inf = tg_kkt_fold(inf, -cj);
+        dinf = tg_kkt_fold(dinf, -rj);
+        comp = tg_kkt_fold(comp, fabs(rj * cj));
+    }
+    int k0 = 0;
+    tg_wargmax(st, k0); tg_wargmax(inf, k0); tg_wargmax(dinf, k0); tg_wargmax(comp, k0);
+    if (lane == 0) { kkt[0] = st; kkt[1] = inf; kkt[2] = dinf; kkt[3] = comp; }
+    TG_SYNC();
+}
+
 
 #endif  // TG_SQP_H

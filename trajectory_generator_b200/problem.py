@@ -41,6 +41,26 @@ class Layout:
             Layout._cache[key] = fields
         self.__dict__.update(fields)
 
+    # constraint row blocks in SLSQP row order: (name, first-row field, row-count field, kind)
+    _ROW_BLOCKS = (("start", "r_start", "n_start", "eq"), ("end", "r_end", "n_end", "eq"),
+                   ("start_derivatives", "r_sder", "n_sder", "eq"), ("end_derivatives", "r_eder", "n_eder", "eq"),
+                   ("intermediate_locations", "r_iwl", "n_iwl", "eq"), ("intermediate_velocities", "r_iwv", "n_iwv", "eq"),
+                   ("derivative_bounds", "r_db", "n_db", "ineq"), ("tangential_lower", "r_tanl", "n_tan", "ineq"),
+                   ("tangential_upper", "r_tanu", "n_tan", "ineq"), ("turning", "r_turn", "n_turn", "ineq"),
+                   ("corridor_lower", "r_sfcl", "n_sfc", "ineq"), ("corridor_upper", "r_sfcu", "n_sfc", "ineq"),
+                   ("obstacles", "r_obs", "n_obs", "ineq"))
+
+    def row_blocks(self):
+        """The non-empty constraint row blocks in row order, as (name, start, stop, "eq" | "ineq"): which rows of the
+        constraint values and of the multipliers (batch.solve(..., multipliers=True)) belong to which constraint.  They
+        tile [0, m); the equality blocks come first and end at meq."""
+        out = []
+        for name, r, cnt, kind in self._ROW_BLOCKS:
+            start, count = getattr(self, r), getattr(self, cnt)
+            if count:
+                out.append((name, start, start + count, kind))
+        return out
+
 
 class PackedProblem:
     def __init__(self, spec, par, x0, xl, xu):

@@ -17,12 +17,17 @@ from .problem import PackedGroup, pack_problem, pack_problems
 class TrajectoryResult:
     """Per-problem solver outcome that the reference keeps internal (OptimizeResult.status / nit / fun)."""
 
-    def __init__(self, control_points, scale_factor, is_violation, status, nit, fun, x, start=0, max_violation=None):
+    def __init__(self, control_points, scale_factor, is_violation, status, nit, fun, x, start=0, max_violation=None,
+                 multipliers=None, kkt=None):
         """start: the multi-start start that won (0 without multi-start); max_violation: its true maximum constraint
-        violation (computed by multi-start solves only, else None)."""
+        violation (computed by multi-start solves only, else None).  multipliers [m] / kkt [4]: the KKT multipliers of
+        the last QP in constraint row order (scipy's OptimizeResult.multipliers; Layout.row_blocks names the rows) and
+        the first-order optimality certificate (batch.KKT_FIELDS), with TrajectoryGenerator(..., multipliers=True)
+        only, else None."""
         self.control_points, self.scale_factor, self.is_violation = control_points, scale_factor, is_violation
         self.status, self.nit, self.fun, self.x = status, nit, fun, x
         self.start, self.max_violation = start, max_violation
+        self.multipliers, self.kkt = multipliers, kkt
         self.success = status == 0
 
     def __iter__(self):      # unpacks like the reference's return tuple
@@ -31,7 +36,7 @@ class TrajectoryResult:
 
 class TrajectoryGenerator:
     def __init__(self, dimension: int, jacobian: str = "fd", maxiter: int = 100, ftol: float = 1e-6, starts: int = 1,
-                 seed: int = 0):
+                 seed: int = 0, multipliers: bool = False):
         """jacobian: "fd" (default) forms derivatives on the GPU exactly as scipy does for the reference (2-point
         forward differences, h = 1.49e-8, bound-aware), so the iterates follow the reference's and the converged
         control points agree within 1e-5 wherever the reference reproduces itself to that level; "analytic" uses
@@ -39,13 +44,17 @@ class TrajectoryGenerator:
         maxiter / ftol default to scipy's SLSQP defaults, which is what the reference runs with
         (TG/trajectory_generator.py:85).
         starts > 1: every problem is solved from `starts` seeded starts on the device (start 0 is the usual one) and the
-        best converged feasible result is kept (batch.solve_mixed_multistart; DESIGN.md §4 *Multi-start*)."""
+        best converged feasible result is kept (batch.solve_mixed_multistart; DESIGN.md §4 *Multi-start*).
+        multipliers: every TrajectoryResult also carries the KKT multipliers and the optimality certificate
+        (DESIGN.md §4 *Multipliers and the KKT certificate*); the groups are then solved through the device entry
+        points."""
         if int(starts) < 1:
             raise ValueError("starts must be at least 1")
         self._dimension = dimension
         self._order = 3
         self._jacobian, self._maxiter, self._ftol = jacobian, maxiter, ftol
         self._starts, self._seed = int(starts), int(seed)
+        self._multipliers = bool(multipliers)
         self.last_result = None
 
     # ---- reference API ---------------------------------------------------------------------------
@@ -116,7 +125,7 @@ class TrajectoryGenerator:
 
     def _solve_groups(self, groups, results, offset):
         """one library call for the groups (shapes) of a chunk; results[offset + index] are filled in"""
-        if self._starts > 1:
+        if self._starts > 1 or self._multipliers:
             return self._solve_groups_multistart(groups, results, offset)
         buckets = [(g.spec, g.par, g.x0) for g in groups]
         if len(buckets) == 1:
@@ -134,20 +143,29 @@ class TrajectoryGenerator:
         return results
 
     def _solve_groups_multistart(self, groups, results, offset):
-        """the groups moved to the current CUDA device and solved from self._starts starts each"""
+        """the groups moved to the current CUDA device and solved from self._starts starts each (one start: an ordinary
+        device solve, batch.solve / solve_mixed)"""
         import torch
         dev = torch.device("cuda", torch.cuda.current_device())
         buckets = [(g.spec, torch.from_numpy(np.ascontiguousarray(g.par)).to(dev),
                     torch.from_numpy(np.ascontiguousarray(g.x0)).to(dev)) for g in groups]
-        outs = batch.solve_mixed_multistart(buckets, self._starts, self._seed, maxiter=self._maxiter, ftol=self._ftol,
-                                            jacobian=self._jacobian)
+        if self._starts > 1:
+            outs = batch.solve_mixed_multistart(buckets, self._starts, self._seed, maxiter=self._maxiter, ftol=self._ftol,
+                                                jacobian=self._jacobian, multipliers=self._multipliers)
+        elif len(buckets) == 1:
+            outs = [batch.solve(*buckets[0], maxiter=self._maxiter, ftol=self._ftol, jacobian=self._jacobian,
+                                multipliers=True)]
+        else:
+            outs = batch.solve_mixed(buckets, self._maxiter, self._ftol, self._jacobian, multipliers=True)
         for g, out in zip(groups, outs):
             lay, idx = g.layout, g.indices
             out = {k: v.cpu().numpy() for k, v in out.items()}
             xs = out["x"]
             cps_all = xs[:, :lay.d * lay.N].reshape(len(idx), lay.d, lay.N).copy()
             for k, i in enumerate(idx.tolist()):
-                results[offset + i] = TrajectoryResult(cps_all[k], float(xs[k, lay.ia]), bool(out["violation"][k]),
-                                                       int(out["status"][k]), int(out["nit"][k]), float(out["f"][k]), xs[k],
-                                                       int(out["best_start"][k]), float(out["max_violation"][k]))
+                results[offset + i] = TrajectoryResult(
+                    cps_all[k], float(xs[k, lay.ia]), bool(out["violation"][k]), int(out["status"][k]), int(out["nit"][k]),
+                    float(out["f"][k]), xs[k], int(out["best_start"][k]) if "best_start" in out else 0,
+                    float(out["max_violation"][k]) if "max_violation" in out else None,
+                    out["lam"][k] if self._multipliers else None, out["kkt"][k] if self._multipliers else None)
         return results
