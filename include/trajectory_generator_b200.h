@@ -159,6 +159,33 @@ int tg_multistart_select(const int *spec, int B, int K, const double *par, const
                          double *max_violation, void *stream);
 
 /*
+ * Post-solve polish (opt-in; csrc/tg_polish.h, DESIGN.md §4 *Polish*).  For every problem with status[b] == 0, a few
+ * safeguarded Newton steps on the KKT system of the solve's final active set -- the equality rows, the inequality rows
+ * with lam_j > 0 and the variables at a bound -- with the exact Lagrangian Hessian (central differences of the analytic
+ * derivatives, also after a finite-difference solve).  Inputs are the outputs of tg_solve_batch_kkt: x[B*n], f[B],
+ * status[B], violation[B], lam[B*m], kkt[B*4].  A row whose polished point passes the final guard (finite; maximum
+ * violation <= max(input's, 1e-8); l1 merit not larger; stationarity, with analytic derivatives, smaller; dual
+ * infeasibility <= 1e-8 max(1, max|lam|)) gets x, f, violation, lam (the working set's least-squares multipliers in row
+ * order, zeros elsewhere) and kkt recomputed at the new point with tg_solve_batch_kkt's definitions and analytic
+ * derivatives; every other row keeps its values bit for bit.  status and nit are not changed.
+ *   polish_status[B]  0 polished (stationarity <= tol max(1, max|g|)), 1 improved (maxiter reached, guard held),
+ *                     2 rejected (guard failed), 3 degenerate (more working-set rows than free variables, or a
+ *                     rank-deficient working set), 4 skipped (status != 0), 5 nonfinite
+ *   polish_iters[B]   Newton iterations taken (a working-set drop counts as one)
+ * Device pointers.  ws: tg_polish_workspace_bytes(spec, B) bytes (0 for shapes whose scratch fits in shared memory,
+ * then ws may be NULL).  Returns 0, or an error code with tg_last_error() (NULL required pointer, no device,
+ * workspace too small).
+ */
+int tg_polish_batch(const int *spec, int B, const double *par, double *x, double *f, const int *status, int *violation,
+                    double *lam, double *kkt, int *polish_status, int *polish_iters, int maxiter, double tol, void *ws,
+                    size_t ws_bytes, void *stream);
+size_t tg_polish_workspace_bytes(const int *spec, int B);
+/* the polish's launch plan on the current device: out[0] lanes per problem, [1] far placement (scratch in workspace
+ * slots), [2] lane groups per CTA, [3] CTAs, [4] KiB of scratch per problem; returns the count (5) or -error code.
+ * TG_POLISH_FAR=1 forces the far placement, TG_GENERIC_KERNELS the generic instantiations. */
+int tg_polish_plan_info(const int *spec, int B, int *out, int cap);
+
+/*
  * Output sampling of a batch of cubic trajectories (SURVEY.md 8(f) f1), device pointers:
  *   mode 0: matrix_bspline_evaluation_for_dataset / matrix_bspline_derivative_evaluation_for_dataset
  *           (TG/matrix_evaluation.py:5-33, 104-135): num_points samples over the N-3 intervals of every trajectory;

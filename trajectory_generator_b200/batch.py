@@ -11,6 +11,8 @@ host-buffer (numpy, copies inside the C call) variants of
 Every solve entry point takes ``multipliers=False``; with True its result also holds ``lam`` [B, m], the KKT
 multipliers of the last QP in constraint row order (scipy's ``OptimizeResult.multipliers``; ``Layout.row_blocks`` names
 the rows), and ``kkt`` [B, 4], the first-order optimality certificate at the returned x (KKT_FIELDS; DESIGN.md §4).
+``polish=True`` (implies multipliers) runs the post-solve polish on the converged rows (``polish``; DESIGN.md §4
+*Polish*) and adds ``polish_status`` and ``polish_iters``.
 
 PyTorch is used only to own device memory and streams.
 """
@@ -24,6 +26,10 @@ from .problem import Layout
 JACOBIAN_MODES = {"analytic": 0, "fd": 1}     # "fd": scipy's forward differences emulated on the GPU
 # entries of `kkt` (include/trajectory_generator_b200.h, tg_solve_batch_kkt): absolute, NaN = +inf
 KKT_FIELDS = ("stationarity", "infeasibility", "dual_infeasibility", "complementarity")
+# codes of `polish_status` (include/trajectory_generator_b200.h, tg_polish_batch)
+POLISH_STATUS = {0: "polished", 1: "improved", 2: "rejected", 3: "degenerate", 4: "skipped", 5: "nonfinite"}
+POLISH_MAXITER = 8      # Newton iterations of the polish (DESIGN.md §4 *Polish*: the choice and its measurement)
+POLISH_TOL = 1e-8       # stationarity target, relative to max(1, max|g|)
 
 
 def _torch():
@@ -119,10 +125,12 @@ def _kkt_outputs(torch, lay, B, dev):
                 kkt=torch.empty((B, 4), dtype=torch.float64, device=dev))
 
 
-def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=None, fused=False, multipliers=False):
+def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=None, fused=False, multipliers=False,
+          polish=False):
     """Device-resident M2 solve.  x [B,n] is overwritten with the optimised variables.
     Returns dict(x, f, status, nit, violation) of CUDA tensors; with multipliers=True also lam [B, m] and kkt [B, 4]
-    (tg_solve_batch_kkt), new tensors of every call.
+    (tg_solve_batch_kkt), new tensors of every call; with polish=True (implies multipliers) the converged rows polished
+    (``polish``) plus polish_status and polish_iters.
     fused=False (default): lock-step stage kernels over the whole batch; fused=True: one persistent kernel in
     which each warp runs a whole solve (same arithmetic, kept for comparison)."""
     torch = _torch()
@@ -137,6 +145,7 @@ def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=Non
     if not (par.is_contiguous() and x.is_contiguous()) or par.shape != (B, lay.P) or x.shape != (B, lay.n):
         raise ValueError("par [B, %d] and x [B, %d] must be contiguous tensors of the descriptor's shape" % (lay.P, lay.n))
     dev = x.device
+    multipliers = multipliers or polish
     buf = buffers if buffers is not None else SolveBuffers(spec, B, dev)
     if buf.B < B or not np.array_equal(buf.spec, np.ascontiguousarray(spec, dtype=np.int32)) or buf.ws.device != dev:
         raise ValueError("the SolveBuffers were made for another shape, a smaller batch or another device")
@@ -149,7 +158,57 @@ def solve(spec, par, x, maxiter=100, ftol=1e-6, jacobian="analytic", buffers=Non
         else:
             rc = _native.lib().tg_solve_batch(*args)
     _native.check(rc, "tg_solve_batch_kkt" if multipliers else "tg_solve_batch")
-    return dict(x=x, f=buf.f, status=buf.status, nit=buf.nit, violation=buf.violation, **extra)
+    res = dict(x=x, f=buf.f, status=buf.status, nit=buf.nit, violation=buf.violation, **extra)
+    return _polish(spec, par, res) if polish else res
+
+
+def polish(spec, par, result, maxiter=POLISH_MAXITER, tol=POLISH_TOL):
+    """Post-solve polish (tg_polish_batch; DESIGN.md §4 *Polish*) of a result dict of ``solve(..., multipliers=True)``:
+    every row with status 0 gets up to `maxiter` safeguarded Newton steps on the KKT system of the solve's final active
+    set with the exact Lagrangian Hessian (analytic derivatives, whatever Jacobian mode the solve used).  x, f,
+    violation, lam and kkt are updated in place where the polished point passes the final guard and kept bit for bit
+    elsewhere; status and nit stay.  Adds polish_status [B] (codes in POLISH_STATUS) and polish_iters [B]; returns
+    `result`.  par [B, P]: the rows the solve ran with."""
+    torch = _torch()
+    if "lam" not in result or "kkt" not in result:
+        raise ValueError("polish() needs the multipliers of the solve: solve(..., multipliers=True)")
+    x = result["x"]
+    lay, B = _check_device_rows("polish()", spec, par, x)
+    dev = x.device
+    for k, dtype in (("f", torch.float64), ("status", torch.int32), ("violation", torch.int32), ("lam", torch.float64),
+                     ("kkt", torch.float64)):
+        t = result[k]
+        if not t.is_cuda or t.device != dev or t.dtype != dtype or not t.is_contiguous() or t.shape[0] != B:
+            raise ValueError("polish(): result[%r] must be a contiguous %s CUDA tensor with %d rows" % (k, dtype, B))
+    result["polish_status"] = torch.empty(B, dtype=torch.int32, device=dev)
+    result["polish_iters"] = torch.empty(B, dtype=torch.int32, device=dev)
+    spec, sp = _native.spec_ptr(spec)
+    L = _native.lib()
+    with torch.cuda.device(dev):
+        nbytes = L.tg_polish_workspace_bytes(sp, B)
+        ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        rc = L.tg_polish_batch(sp, B, _ptr(par), _ptr(x), _ptr(result["f"]), _ptr(result["status"]),
+                               _ptr(result["violation"]), _ptr(result["lam"]), _ptr(result["kkt"]),
+                               _ptr(result["polish_status"]), _ptr(result["polish_iters"]), int(maxiter), float(tol),
+                               _ptr(ws), ws.numel(), _stream(torch, dev))
+    _native.check(rc, "tg_polish_batch")
+    return result
+
+
+_polish = polish        # (the solve entry points' `polish` argument shadows the name)
+
+
+POLISH_PLAN_FIELDS = ("lanes", "far", "groups", "ctas", "kib_per_problem")
+
+
+def polish_plan(spec, B):
+    """Launch plan of the polish of B problems of this shape on the current device (tg_polish_plan_info): a dict keyed
+    by POLISH_PLAN_FIELDS."""
+    spec, sp = _native.spec_ptr(spec)
+    out = np.zeros(len(POLISH_PLAN_FIELDS), dtype=np.int32)
+    cnt = _native.lib().tg_polish_plan_info(sp, int(B), out.ctypes.data_as(_native._I32), out.size)
+    _native.check(-cnt if cnt < 0 else 0, "tg_polish_plan_info")
+    return {k: int(v) for k, v in zip(POLISH_PLAN_FIELDS, out)}
 
 
 def _np_ptr(a):
@@ -242,14 +301,16 @@ def solve_mixed_host(buckets, maxiter=100, ftol=1e-6, jacobian="analytic"):
     return outs
 
 
-def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic", multipliers=False):
+def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic", multipliers=False, polish=False):
     """Device-resident M2 solve of problems of DIFFERENT shapes in one call (tg_solve_mixed_batch).
     buckets: list of (spec, par [Bk, P], x [Bk, n]) CUDA tensors; x is overwritten with the solution.  The buckets run
     concurrently on internal streams that fork from and join the current stream.  Returns one dict(x, f, status, nit,
     violation) of CUDA tensors per bucket; with multipliers=True each also holds lam [Bk, m] and kkt [Bk, 4]
-    (tg_solve_mixed_batch_kkt)."""
+    (tg_solve_mixed_batch_kkt); polish=True (implies multipliers) polishes every bucket afterwards on the current stream.
+    """
     torch = _torch()
     L = _native.lib()
+    multipliers = multipliers or polish
     nb = len(buckets)
     if nb == 0:
         return []
@@ -289,6 +350,9 @@ def solve_mixed(buckets, maxiter=100, ftol=1e-6, jacobian="analytic", multiplier
     with torch.cuda.device(dev):
         rc = fn(*args, ptrs["lam"], ptrs["kkt"]) if multipliers else fn(*args)
     _native.check(rc, name)
+    if polish:
+        for (spec, par, _), out in zip(buckets, outs):
+            _polish(spec, par, out)
     return outs
 
 
@@ -366,15 +430,17 @@ def multistart_select(spec, par, sol, starts, tol=MULTISTART_TOL, out=None):
 
 
 def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100,
-                           ftol=1e-6, jacobian="analytic", return_all=False, multipliers=False):
+                           ftol=1e-6, jacobian="analytic", return_all=False, multipliers=False, polish=False):
     """Multi-start solve of problems of one or several shapes: buckets = list of (spec, par [Bk, P], x0 [Bk, n]) CUDA
     tensors (x0 is not modified).  Per bucket: expand -> solve -> select on the current stream, in pieces of at most
     MULTISTART_ROWS expanded rows; the pieces of several shapes go through one ``solve_mixed`` call.  Returns one dict
     per bucket: the B-row dict of ``solve`` plus best_start and max_violation (the winner's true maximum violation);
     with return_all, also "all": the K per-start results, dict(x [B, K, n], f, status, nit, violation,
     max_violation [B, K]).  multipliers=True adds the winner's lam [B, m] and kkt [B, 4] (and every start's,
-    [B, K, m] and [B, K, 4], under "all")."""
+    [B, K, m] and [B, K, 4], under "all").  polish=True (implies multipliers) polishes the winners after the selection
+    (the rows under "all" stay as the solve left them); a replaced winner's max_violation is its polished kkt[1]."""
     torch = _torch()
+    multipliers = multipliers or polish
     K = int(starts)
     if K < 1:
         raise ValueError("starts must be at least 1")
@@ -428,17 +494,23 @@ def solve_mixed_multistart(buckets, starts, seed=0, spread=MULTISTART_SPREAD, to
             if return_all:
                 for k in ("x", "f", "status", "nit", "violation") + (("lam", "kkt") if multipliers else ()):
                     res["all"][k][lo:hi] = sol[k].view(res["all"][k][lo:hi].shape)
-    for res in outs:
+    for (spec, par, _), res in zip(buckets, outs):
         mv = res.pop("start_max_violation")
         res["max_violation"] = mv.gather(1, res["best_start"].long()[:, None])[:, 0]
         if return_all:
             res["all"]["max_violation"] = mv
+        if polish:
+            rows = {k: res[k] for k in ("x", "f", "status", "violation", "lam", "kkt")}
+            _polish(spec, par, rows)
+            res["polish_status"], res["polish_iters"] = rows["polish_status"], rows["polish_iters"]
+            replaced = res["polish_status"] <= 1
+            res["max_violation"] = torch.where(replaced, res["kkt"][:, 1], res["max_violation"])
     return outs
 
 
 def solve_multistart(spec, par, x0, starts, seed=0, spread=MULTISTART_SPREAD, tol=MULTISTART_TOL, maxiter=100, ftol=1e-6,
-                     jacobian="analytic", return_all=False, multipliers=False):
+                     jacobian="analytic", return_all=False, multipliers=False, polish=False):
     """Multi-start solve of B problems of one shape (see ``solve_mixed_multistart``).  starts = 1 returns exactly what
     ``solve`` returns for x0 (start 0 is x0 itself), plus best_start = 0 and max_violation."""
     return solve_mixed_multistart([(spec, par, x0)], starts, seed, spread, tol, maxiter, ftol, jacobian, return_all,
-                                  multipliers)[0]
+                                  multipliers, polish)[0]

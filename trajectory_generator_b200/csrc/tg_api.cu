@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "tg_sqp.h"
+#include "tg_polish.h"
 #include "tg_shape.h"
 #include "../../include/trajectory_generator_b200.h"
 
@@ -932,6 +933,86 @@ extern "C" int tg_multistart_select(const int *spec, int B, int K, const double 
     cudaError_t e = launchers[tg_lanes_index(gs)](a);
     g_launches++;
     if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_select_kernel launch", e);
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
+// post-solve polish (tg_kernels_polish.inc): lanes from the shape, lane groups per CTA from shared memory; shapes whose
+// scratch does not fit (or TG_POLISH_FAR=1) take it from workspace slots, one per lane group of a grid capped at
+// TG_FAR_CTAS_PER_SM CTAs per SM and at TG_POLISH_FAR_BYTES of slots.  Near and far use the same lanes, so that they
+// compute the same bits.
+// ---------------------------------------------------------------------------
+#define TG_POLISH_FAR_BYTES ((size_t)4 << 30)
+struct TgPolishPlan {
+    int fix, lanes, far, groups, grid;
+    size_t per_bytes, smem, ws_bytes;
+};
+
+static int tg_plan_polish(const TgShape &S, int B, TgPolishPlan *P)
+{
+    int rc = tg_device_check();
+    if (rc) return rc;
+    const TgLayout &L = S.L;
+    P->fix = tg_plan_fix(S);
+    // (the dense linear algebra strides over the free variables: a warp once they are more than 32)
+    P->lanes = L.n > 32 ? 32 : tg_default_gs(L);
+    P->per_bytes = tg_polish_group_doubles(L) * sizeof(double);
+    const size_t fit = ((size_t)g_smem_optin - 1024) / P->per_bytes;
+    const char *v = getenv("TG_POLISH_FAR");
+    P->far = fit == 0 || (v && atoi(v) != 0);
+    P->groups = TG_CTA_THREADS / P->lanes;
+    if (!P->far && fit < (size_t)P->groups) P->groups = (int)fit;
+    size_t grid = ((size_t)B + P->groups - 1) / P->groups, cap = (size_t)g_sm_count * 32;
+    if (P->far) {
+        const size_t cta_bytes = (size_t)P->groups * P->per_bytes, budget = TG_POLISH_FAR_BYTES / cta_bytes;
+        cap = (size_t)g_sm_count * TG_FAR_CTAS_PER_SM;
+        if (budget < cap) cap = budget > 0 ? budget : 1;
+    }
+    P->grid = (int)(grid < cap ? grid : cap);
+    P->smem = P->far ? 0 : (size_t)P->groups * P->per_bytes;
+    P->ws_bytes = P->far ? (((size_t)P->grid * P->groups * P->per_bytes) + 255) & ~(size_t)255 : 0;
+    return 0;
+}
+
+extern "C" size_t tg_polish_workspace_bytes(const int *spec, int B)
+{
+    TgShape S;
+    TgPolishPlan P;
+    if (tg_make_shape(spec, &S) || tg_plan_polish(S, B > 0 ? B : 1, &P)) return 0;
+    return P.ws_bytes;
+}
+
+extern "C" int tg_polish_plan_info(const int *spec, int B, int *out, int cap)
+{
+    TgShape S;
+    TgPolishPlan P;
+    int rc = tg_make_shape(spec, &S);
+    if (!rc) rc = tg_plan_polish(S, B > 0 ? B : 1, &P);
+    if (rc) return -rc;
+    const int v[5] = {P.lanes, P.far, P.groups, P.grid, (int)(P.per_bytes >> 10)};
+    for (int i = 0; i < 5 && out && i < cap; i++) out[i] = v[i];
+    return 5;
+}
+
+extern "C" int tg_polish_batch(const int *spec, int B, const double *par, double *x, double *f, const int *status,
+                               int *violation, double *lam, double *kkt, int *polish_status, int *polish_iters,
+                               int maxiter, double tol, void *ws, size_t ws_bytes, void *stream)
+{
+    TgShape S;
+    int rc = tg_make_shape(spec, &S);
+    if (rc) return rc;
+    if (B <= 0) return 0;
+    if (!par || !x || !f || !status || !violation || !lam || !kkt || !polish_status || !polish_iters)
+        return tg_fail(1, "tg_polish_batch: NULL argument");
+    TgPolishPlan P;
+    if ((rc = tg_plan_polish(S, B, &P))) return rc;
+    if (P.ws_bytes && (!ws || ws_bytes < P.ws_bytes)) return tg_fail(4, "workspace too small (see tg_polish_workspace_bytes)");
+    const TgPolishLaunch a = {S, B, par, x, f, status, violation, lam, kkt, polish_status, polish_iters, maxiter, tol,
+                              P.far ? (double *)ws : nullptr, P.fix, P.grid, P.groups, P.smem, (cudaStream_t)stream};
+    static cudaError_t (*const launchers[3])(const TgPolishLaunch &) = {tg_launch_polish_g8, tg_launch_polish_g16, tg_launch_polish_g32};
+    cudaError_t e = launchers[tg_lanes_index(P.lanes)](a);
+    g_launches++;
+    if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_polish_kernel launch", e);
     return 0;
 }
 

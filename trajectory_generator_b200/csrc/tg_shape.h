@@ -170,6 +170,26 @@ struct TgSelectLaunch {
 };
 cudaError_t tg_launch_select_g8(const TgSelectLaunch &a), tg_launch_select_g16(const TgSelectLaunch &a),
     tg_launch_select_g32(const TgSelectLaunch &a);
+// Post-solve polish kernel (tg_kernels_polish.inc, planned by tg_plan_polish): `groups` lane groups per CTA, each with
+// tg_polish_group_doubles of scratch in `smem` (far == nullptr) or in its slot of `far`
+struct TgPolishLaunch {
+    TgShape S;
+    int B;
+    const double *par;
+    double *x, *f;
+    const int *status;
+    int *violation;
+    double *lam, *kkt;
+    int *polish_status, *polish_iters;
+    int maxiter;
+    double tol;
+    double *far;
+    int fix, grid, groups;
+    size_t smem;
+    cudaStream_t st;
+};
+cudaError_t tg_launch_polish_g8(const TgPolishLaunch &a), tg_launch_polish_g16(const TgPolishLaunch &a),
+    tg_launch_polish_g32(const TgPolishLaunch &a);
 // Multi-start expansion (tg_multistart.cu)
 cudaError_t tg_launch_multistart_expand(const TgLayout &L, int B, int K, const double *par, const double *x0,
                                         unsigned long long seed, double spread, double *par_out, double *x_out,

@@ -18,16 +18,18 @@ class TrajectoryResult:
     """Per-problem solver outcome that the reference keeps internal (OptimizeResult.status / nit / fun)."""
 
     def __init__(self, control_points, scale_factor, is_violation, status, nit, fun, x, start=0, max_violation=None,
-                 multipliers=None, kkt=None):
+                 multipliers=None, kkt=None, polish_status=None):
         """start: the multi-start start that won (0 without multi-start); max_violation: its true maximum constraint
         violation (computed by multi-start solves only, else None).  multipliers [m] / kkt [4]: the KKT multipliers of
         the last QP in constraint row order (scipy's OptimizeResult.multipliers; Layout.row_blocks names the rows) and
         the first-order optimality certificate (batch.KKT_FIELDS), with TrajectoryGenerator(..., multipliers=True)
-        only, else None."""
+        only, else None.  polish_status: the post-solve polish's code (batch.POLISH_STATUS) with
+        TrajectoryGenerator(..., polish=True) only, else None."""
         self.control_points, self.scale_factor, self.is_violation = control_points, scale_factor, is_violation
         self.status, self.nit, self.fun, self.x = status, nit, fun, x
         self.start, self.max_violation = start, max_violation
         self.multipliers, self.kkt = multipliers, kkt
+        self.polish_status = polish_status
         self.success = status == 0
 
     def __iter__(self):      # unpacks like the reference's return tuple
@@ -36,7 +38,7 @@ class TrajectoryResult:
 
 class TrajectoryGenerator:
     def __init__(self, dimension: int, jacobian: str = "fd", maxiter: int = 100, ftol: float = 1e-6, starts: int = 1,
-                 seed: int = 0, multipliers: bool = False):
+                 seed: int = 0, multipliers: bool = False, polish: bool = False):
         """jacobian: "fd" (default) forms derivatives on the GPU exactly as scipy does for the reference (2-point
         forward differences, h = 1.49e-8, bound-aware), so the iterates follow the reference's and the converged
         control points agree within 1e-5 wherever the reference reproduces itself to that level; "analytic" uses
@@ -47,14 +49,17 @@ class TrajectoryGenerator:
         best converged feasible result is kept (batch.solve_mixed_multistart; DESIGN.md §4 *Multi-start*).
         multipliers: every TrajectoryResult also carries the KKT multipliers and the optimality certificate
         (DESIGN.md §4 *Multipliers and the KKT certificate*); the groups are then solved through the device entry
-        points."""
+        points.
+        polish: the converged problems are polished on the device after the solve (batch.polish; DESIGN.md §4 *Polish*):
+        the results hold the polished x, and multipliers, kkt and polish_status are filled in (implies multipliers)."""
         if int(starts) < 1:
             raise ValueError("starts must be at least 1")
         self._dimension = dimension
         self._order = 3
         self._jacobian, self._maxiter, self._ftol = jacobian, maxiter, ftol
         self._starts, self._seed = int(starts), int(seed)
-        self._multipliers = bool(multipliers)
+        self._polish = bool(polish)
+        self._multipliers = bool(multipliers) or self._polish
         self.last_result = None
 
     # ---- reference API ---------------------------------------------------------------------------
@@ -151,12 +156,14 @@ class TrajectoryGenerator:
                     torch.from_numpy(np.ascontiguousarray(g.x0)).to(dev)) for g in groups]
         if self._starts > 1:
             outs = batch.solve_mixed_multistart(buckets, self._starts, self._seed, maxiter=self._maxiter, ftol=self._ftol,
-                                                jacobian=self._jacobian, multipliers=self._multipliers)
+                                                jacobian=self._jacobian, multipliers=self._multipliers,
+                                                polish=self._polish)
         elif len(buckets) == 1:
             outs = [batch.solve(*buckets[0], maxiter=self._maxiter, ftol=self._ftol, jacobian=self._jacobian,
-                                multipliers=True)]
+                                multipliers=True, polish=self._polish)]
         else:
-            outs = batch.solve_mixed(buckets, self._maxiter, self._ftol, self._jacobian, multipliers=True)
+            outs = batch.solve_mixed(buckets, self._maxiter, self._ftol, self._jacobian, multipliers=True,
+                                     polish=self._polish)
         for g, out in zip(groups, outs):
             lay, idx = g.layout, g.indices
             out = {k: v.cpu().numpy() for k, v in out.items()}
@@ -167,5 +174,6 @@ class TrajectoryGenerator:
                     cps_all[k], float(xs[k, lay.ia]), bool(out["violation"][k]), int(out["status"][k]), int(out["nit"][k]),
                     float(out["f"][k]), xs[k], int(out["best_start"][k]) if "best_start" in out else 0,
                     float(out["max_violation"][k]) if "max_violation" in out else None,
-                    out["lam"][k] if self._multipliers else None, out["kkt"][k] if self._multipliers else None)
+                    out["lam"][k] if self._multipliers else None, out["kkt"][k] if self._multipliers else None,
+                    int(out["polish_status"][k]) if self._polish else None)
         return results
