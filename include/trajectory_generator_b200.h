@@ -186,6 +186,32 @@ size_t tg_polish_workspace_bytes(const int *spec, int B);
 int tg_polish_plan_info(const int *spec, int B, int *out, int cap);
 
 /*
+ * Parameter sensitivities of converged solves (opt-in; csrc/tg_sens.h, DESIGN.md §4 *Sensitivities*).  For every
+ * problem with status[b] == 0 and upstream gradients x_bar[b*n] (of a scalar loss with respect to x) and f_bar[b] (with
+ * respect to f; f_bar == NULL means zeros), par_bar[b*P] = d loss / d par from one adjoint solve of the KKT system of
+ * the working set -- the equality rows and the inequality rows with lam_j > 0, the variables at a bound held fixed --
+ * with the exact Lagrangian Hessian (analytic derivatives) and the least-squares multipliers at x; the parameter
+ * derivatives of the constraints, linear rows included, by central differences.  Inputs are the outputs of
+ * tg_solve_batch_kkt, possibly polished (tg_polish_batch): x[B*n], status[B], lam[B*m].
+ *   sens_status[B]  0 ok, 1 nonstrict (an inequality row is weakly active: the derivative holds the working set fixed
+ *                   and is one-sided), 2 inexact (stationarity with lam and analytic derivatives > tol max(1, max|g|),
+ *                   or a negative least-squares multiplier on an inequality row) -- par_bar computed; 3 degenerate
+ *                   (more working-set rows than free variables, or a rank-deficient working set), 4 skipped
+ *                   (status != 0), 5 nonfinite, 6 indefinite (the reduced Hessian has no Cholesky factor: no unique
+ *                   derivative) -- par_bar row zero
+ * Device pointers, stream-ordered, no host synchronisation.  ws: tg_sens_workspace_bytes(spec, B) bytes (0 for shapes
+ * whose scratch fits in shared memory, then ws may be NULL).  Returns 0, or an error code with tg_last_error() (NULL
+ * required pointer, no device, workspace too small).
+ */
+int tg_sens_batch(const int *spec, int B, const double *par, const double *x, const int *status, const double *lam,
+                  const double *x_bar, const double *f_bar, double *par_bar, int *sens_status, double tol, void *ws,
+                  size_t ws_bytes, void *stream);
+size_t tg_sens_workspace_bytes(const int *spec, int B);
+/* the sensitivities' launch plan: the five fields of tg_polish_plan_info; TG_POLISH_FAR=1 and TG_GENERIC_KERNELS act
+ * on it too. */
+int tg_sens_plan_info(const int *spec, int B, int *out, int cap);
+
+/*
  * Output sampling of a batch of cubic trajectories (SURVEY.md 8(f) f1), device pointers:
  *   mode 0: matrix_bspline_evaluation_for_dataset / matrix_bspline_derivative_evaluation_for_dataset
  *           (TG/matrix_evaluation.py:5-33, 104-135): num_points samples over the N-3 intervals of every trajectory;

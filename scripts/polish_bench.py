@@ -8,9 +8,11 @@ untimed warm-up of each: the solve with multipliers, the polish of a copy of its
 at ftol = 1e-10, maxiter = 400 with multipliers; device time from CUDA events around each call.  Reported: the status-0
 share; over the status-0 problems the stationarity (kkt[0]) median / p99 and the shares <= 1e-6 and <= 1e-8 before and
 after the polish and of the baseline; the polish_status histogram; over the replaced rows the mean change of f and of
-the maximum violation (kkt[1]).  Writes OUTDIR/polish.json and OUTDIR/polish.md with the card's name and power limit
+the maximum violation (kkt[1]); a SHA-256 checksum of the polished outputs (x, f, violation, lam, kkt, polish_status,
+polish_iters), which compares the polish's bits across versions.  Writes OUTDIR/polish.json and OUTDIR/polish.md with the card's name and power limit
 read in the same run."""
 import argparse
+import hashlib
 import json
 import os
 import sys
@@ -63,13 +65,16 @@ def run(bt, jac, repeats):
     bl = {k: v.cpu().numpy() for k, v in bl.items()}
     ok, okb = sol["status"] == 0, bl["status"] == 0
     rep = ok & (pol["polish_status"] <= 1)
+    ck = hashlib.sha256()
+    for k in ("x", "f", "violation", "lam", "kkt", "polish_status", "polish_iters"):
+        ck.update(np.ascontiguousarray(pol[k]).tobytes())
     hist = {batch.POLISH_STATUS[k]: int(np.sum(pol["polish_status"][ok] == k)) for k in range(6) if k != 4}
     return dict(status0=float(ok.mean()), before=_stationarity(sol["kkt"], ok), after=_stationarity(pol["kkt"], ok),
                 polish_status=hist, replaced=int(rep.sum()),
                 mean_df=float(np.mean(pol["f"][rep] - sol["f"][rep])) if rep.any() else 0.0,
                 mean_dviol=float(np.mean(pol["kkt"][rep, 1] - sol["kkt"][rep, 1])) if rep.any() else 0.0,
                 baseline_status0=float(okb.mean()), baseline=_stationarity(bl["kkt"], okb),
-                ms=t)
+                checksum=ck.hexdigest(), ms=t)
 
 
 def main():

@@ -26,9 +26,9 @@ LAYOUT_FIELDS = ("d N nint n ia is0 is1 it0 nws niw meq mineq m r_start n_start 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 # translation units: the host API (+ legacy single-problem kernels) and one unit per (kernel family, lanes per problem)
-UNITS = ["tg_api.cu", "tg_sample.cu", "tg_build.cu", "tg_smooth.cu", "tg_multistart.cu", "tg_solve_fused.cu", "tg_solve_g64.cu"] + ["tg_%s_g%d.cu" % (fam, gs) for fam in ("eval", "solve", "solve_fd", "polish") for gs in (8, 16, 32)]
+UNITS = ["tg_api.cu", "tg_sample.cu", "tg_build.cu", "tg_smooth.cu", "tg_multistart.cu", "tg_solve_fused.cu", "tg_solve_g64.cu"] + ["tg_%s_g%d.cu" % (fam, gs) for fam in ("eval", "solve", "solve_fd", "polish", "sens") for gs in (8, 16, 32)]
 HEADERS = ["tg_sqp.h", "tg_eval.h", "tg_spec.h", "tg_shape.h", "tg_smooth.h", "tg_kernels_eval.inc", "tg_kernels_solve.inc", "tg_polish.h",
-           "tg_kernels_polish.inc"]
+           "tg_kernels_polish.inc", "tg_sens.h", "tg_kernels_sens.inc"]
 
 
 def build_native(force=False, verbose=False, variant=None, extra_flags=()):
@@ -140,6 +140,12 @@ def lib():
         L.tg_polish_workspace_bytes.restype = sz
         L.tg_polish_plan_info.argtypes = [_I32, ctypes.c_int, _I32, ctypes.c_int]
         L.tg_polish_plan_info.restype = ctypes.c_int
+        L.tg_sens_batch.argtypes = [_I32, ctypes.c_int] + [vp] * 8 + [ctypes.c_double, vp, sz, vp]
+        L.tg_sens_batch.restype = ctypes.c_int
+        L.tg_sens_workspace_bytes.argtypes = [_I32, ctypes.c_int]
+        L.tg_sens_workspace_bytes.restype = sz
+        L.tg_sens_plan_info.argtypes = [_I32, ctypes.c_int, _I32, ctypes.c_int]
+        L.tg_sens_plan_info.restype = ctypes.c_int
         for name in ("tg_eval_batch", "tg_linear_rows_batch", "tg_solve_batch", "tg_solve_batch_kkt", "tg_eval_host", "tg_solve_host"):
             getattr(L, name).restype = ctypes.c_int
         _LIB = L

@@ -13,6 +13,9 @@ multipliers of the last QP in constraint row order (scipy's ``OptimizeResult.mul
 the rows), and ``kkt`` [B, 4], the first-order optimality certificate at the returned x (KKT_FIELDS; DESIGN.md §4).
 ``polish=True`` (implies multipliers) runs the post-solve polish on the converged rows (``polish``; DESIGN.md §4
 *Polish*) and adds ``polish_status`` and ``polish_iters``.
+``sensitivity`` turns upstream gradients of x and f of such a result into gradients of the parameter rows, and
+``solve_differentiable`` wraps a solve in a ``torch.autograd.Function`` that does so in its backward (DESIGN.md §4
+*Sensitivities*).
 
 PyTorch is used only to own device memory and streams.
 """
@@ -30,6 +33,9 @@ KKT_FIELDS = ("stationarity", "infeasibility", "dual_infeasibility", "complement
 POLISH_STATUS = {0: "polished", 1: "improved", 2: "rejected", 3: "degenerate", 4: "skipped", 5: "nonfinite"}
 POLISH_MAXITER = 8      # Newton iterations of the polish (DESIGN.md §4 *Polish*: the choice and its measurement)
 POLISH_TOL = 1e-8       # stationarity target, relative to max(1, max|g|)
+# codes of `sens_status` (include/trajectory_generator_b200.h, tg_sens_batch): 0..2 carry par_bar, 3..6 give zeros
+SENS_STATUS = {0: "ok", 1: "nonstrict", 2: "inexact", 3: "degenerate", 4: "skipped", 5: "nonfinite", 6: "indefinite"}
+SENS_TOL = 1e-6         # stationarity above tol max(1, max|g|) makes a row `inexact`
 
 
 def _torch():
@@ -209,6 +215,99 @@ def polish_plan(spec, B):
     cnt = _native.lib().tg_polish_plan_info(sp, int(B), out.ctypes.data_as(_native._I32), out.size)
     _native.check(-cnt if cnt < 0 else 0, "tg_polish_plan_info")
     return {k: int(v) for k, v in zip(POLISH_PLAN_FIELDS, out)}
+
+
+def sensitivity(spec, par, result, x_bar, f_bar=None, tol=SENS_TOL):
+    """Gradients of the parameter rows (tg_sens_batch; DESIGN.md §4 *Sensitivities*) of a result dict that holds the
+    multipliers: any of ``solve``, ``solve_mixed`` or the multi-start solves with ``multipliers=True`` or ``polish=True``.
+    x_bar [B, n] and f_bar [B] (None: zeros) are the gradients of a scalar loss with respect to result["x"] and
+    result["f"]; returns dict(par_bar [B, P], sens_status [B], codes in SENS_STATUS) of new CUDA tensors.  par [B, P]:
+    the rows the solve ran with.  Rows that are not converged, degenerate, indefinite or non-finite get zeros."""
+    torch = _torch()
+    if "lam" not in result or "x" not in result or "status" not in result:
+        raise ValueError("sensitivity() needs the multipliers of the solve: solve(..., multipliers=True)")
+    x = result["x"]
+    lay, B = _check_device_rows("sensitivity()", spec, par, x)
+    dev = x.device
+    checks = [("status", result["status"], torch.int32, (B,)), ("lam", result["lam"], torch.float64, (B, lay.m)),
+              ("x_bar", x_bar, torch.float64, (B, lay.n))]
+    if f_bar is not None:
+        checks.append(("f_bar", f_bar, torch.float64, (B,)))
+    for k, t, dtype, shape in checks:
+        if not t.is_cuda or t.device != dev or t.dtype != dtype or not t.is_contiguous() or tuple(t.shape) != shape:
+            raise ValueError("sensitivity(): %s must be a contiguous %s CUDA tensor of shape %s" % (k, dtype, shape))
+    out = dict(par_bar=torch.empty((B, lay.P), dtype=torch.float64, device=dev),
+               sens_status=torch.empty(B, dtype=torch.int32, device=dev))
+    spec, sp = _native.spec_ptr(spec)
+    L = _native.lib()
+    with torch.cuda.device(dev):
+        nbytes = L.tg_sens_workspace_bytes(sp, B)
+        ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        rc = L.tg_sens_batch(sp, B, _ptr(par), _ptr(x), _ptr(result["status"]), _ptr(result["lam"]), _ptr(x_bar),
+                             _ptr(f_bar), _ptr(out["par_bar"]), _ptr(out["sens_status"]), float(tol), _ptr(ws),
+                             ws.numel(), _stream(torch, dev))
+    _native.check(rc, "tg_sens_batch")
+    return out
+
+
+def sensitivity_plan(spec, B):
+    """Launch plan of the sensitivities of B problems of this shape on the current device (tg_sens_plan_info): a dict
+    keyed by POLISH_PLAN_FIELDS."""
+    spec, sp = _native.spec_ptr(spec)
+    out = np.zeros(len(POLISH_PLAN_FIELDS), dtype=np.int32)
+    cnt = _native.lib().tg_sens_plan_info(sp, int(B), out.ctypes.data_as(_native._I32), out.size)
+    _native.check(-cnt if cnt < 0 else 0, "tg_sens_plan_info")
+    return {k: int(v) for k, v in zip(POLISH_PLAN_FIELDS, out)}
+
+
+_SOLVE_FN = None
+
+
+def _solve_function():
+    """the torch.autograd.Function behind solve_differentiable (made on first use: torch is imported lazily)"""
+    global _SOLVE_FN
+    if _SOLVE_FN is None:
+        torch = _torch()
+
+        class SolveFunction(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, par, x0, spec, maxiter, ftol, jacobian, polish, holder):
+                res = solve(spec, par.detach(), x0.detach().clone(), maxiter=maxiter, ftol=ftol, jacobian=jacobian,
+                            multipliers=True, polish=polish)
+                holder["result"] = res
+                ctx.spec, ctx.status, ctx.lam = spec, res["status"], res["lam"]
+                ctx.save_for_backward(par, res["x"])
+                return res["x"], res["f"]
+
+            @staticmethod
+            @torch.autograd.function.once_differentiable
+            def backward(ctx, grad_x, grad_f):
+                par, x = ctx.saved_tensors
+                if grad_x is None:
+                    grad_x = torch.zeros_like(x)
+                rows = dict(x=x, status=ctx.status, lam=ctx.lam)
+                out = sensitivity(ctx.spec, par, rows, grad_x.contiguous(), None if grad_f is None else grad_f.contiguous())
+                return out["par_bar"], None, None, None, None, None, None, None
+
+        _SOLVE_FN = SolveFunction
+    return _SOLVE_FN
+
+
+def solve_differentiable(spec, par, x0, maxiter=100, ftol=1e-6, jacobian="analytic", polish=True):
+    """``solve(spec, par, x0.clone(), ..., multipliers=True, polish=polish)`` as a differentiable function of par:
+    returns (x [B, n], f [B], result), where result is solve's dict (x and f are the same tensors).  Gradients flow to
+    par through ``sensitivity`` (one adjoint solve per problem); missing upstream gradients count as zeros.  x0 gets no
+    gradient -- a local solution does not depend on its start -- and result's other entries are not differentiable.
+    polish=True by default: SLSQP's own points are rarely stationary, and the derivative assumes stationarity (rows that
+    are not come back `inexact` in the sensitivity statuses).  Rows with status != 0, or with a degenerate or indefinite
+    working set, get zero gradient."""
+    if not (par.is_cuda and x0.is_cuda):
+        raise RuntimeError("solve_differentiable() needs CUDA tensors (there is no CPU path)")
+    holder = {}
+    x, f = _solve_function().apply(par, x0, spec, maxiter, ftol, jacobian, polish, holder)
+    res = holder["result"]
+    res["x"], res["f"] = x, f
+    return x, f, res
 
 
 def _np_ptr(a):

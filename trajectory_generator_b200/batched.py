@@ -8,6 +8,7 @@ the same (shape descriptor, parameter rows, initial variables) ``problem.pack_pr
                         max_velocity=2.0, max_acceleration=5.0, turning=("angular_rate", 1.8),
                         obstacle_centers=ctr, obstacle_radii=rad)
     out = bp.solve()                      # dict(x, f, status, nit, violation); control points: bp.control_points(out)
+    out = bp.solve(differentiable=True)   # x and f differentiable with respect to the tensors given above
     pos = bp.sample(out, num_points=200)  # [B, d, 200]
 
 Every field of a container is supported: terminal waypoints with velocities, directions, accelerations, zero
@@ -175,8 +176,16 @@ class BatchedProblem:
         self.x0 = builder.initial_guess_batch(spec, seq, wseq, initial_scale_factor)
         self.B, self.d, self.N = B, d, N
 
-    def solve(self, jacobian="fd", maxiter=100, ftol=1e-6):
-        """-> dict(x [B,n], f, status, nit, violation) of CUDA tensors (x is a fresh tensor; self.x0 is kept)."""
+    def solve(self, jacobian="fd", maxiter=100, ftol=1e-6, differentiable=False):
+        """-> dict(x [B,n], f, status, nit, violation) of CUDA tensors (x is a fresh tensor; self.x0 is kept).
+        differentiable=True: ``batch.solve_differentiable`` (multipliers and polish included, so the dict also holds
+        lam, kkt, polish_status and polish_iters); x and f are then differentiable, and ``backward()`` reaches the
+        tensors given to the constructor through the parameter rows -- waypoints, velocities, accelerations,
+        directions, bounds given as tensors, obstacle centres and radii.  The corridor block is computed by
+        ``builder.sfc_boxes_batch`` outside autograd: no gradient reaches corridor points or pads (``batch.sensitivity``
+        still returns the gradient of the corridor entries of the rows)."""
+        if differentiable:
+            return tgb.solve_differentiable(self.spec, self.par, self.x0, maxiter=maxiter, ftol=ftol, jacobian=jacobian)[2]
         x = self.x0.clone()
         return tgb.solve(self.spec, self.par, x, maxiter=maxiter, ftol=ftol, jacobian=jacobian)
 

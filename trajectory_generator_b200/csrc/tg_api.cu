@@ -24,7 +24,7 @@
 #include <vector>
 
 #include "tg_sqp.h"
-#include "tg_polish.h"
+#include "tg_sens.h"
 #include "tg_shape.h"
 #include "../../include/trajectory_generator_b200.h"
 
@@ -937,10 +937,11 @@ extern "C" int tg_multistart_select(const int *spec, int B, int K, const double 
 }
 
 // ---------------------------------------------------------------------------
-// post-solve polish (tg_kernels_polish.inc): lanes from the shape, lane groups per CTA from shared memory; shapes whose
-// scratch does not fit (or TG_POLISH_FAR=1) take it from workspace slots, one per lane group of a grid capped at
-// TG_FAR_CTAS_PER_SM CTAs per SM and at TG_POLISH_FAR_BYTES of slots.  Near and far use the same lanes, so that they
-// compute the same bits.
+// post-solve polish (tg_kernels_polish.inc) and parameter sensitivities (tg_kernels_sens.inc): lanes from the shape,
+// lane groups per CTA from shared memory; shapes whose per-problem scratch (`per_doubles`: tg_polish_group_doubles or
+// tg_sens_group_doubles) does not fit (or TG_POLISH_FAR=1) take it from workspace slots, one per lane group of a grid
+// capped at TG_FAR_CTAS_PER_SM CTAs per SM and at TG_POLISH_FAR_BYTES of slots.  Near and far use the same lanes, so
+// that they compute the same bits.
 // ---------------------------------------------------------------------------
 #define TG_POLISH_FAR_BYTES ((size_t)4 << 30)
 struct TgPolishPlan {
@@ -948,7 +949,7 @@ struct TgPolishPlan {
     size_t per_bytes, smem, ws_bytes;
 };
 
-static int tg_plan_polish(const TgShape &S, int B, TgPolishPlan *P)
+static int tg_plan_polish(const TgShape &S, int B, size_t per_doubles, TgPolishPlan *P)
 {
     int rc = tg_device_check();
     if (rc) return rc;
@@ -956,7 +957,7 @@ static int tg_plan_polish(const TgShape &S, int B, TgPolishPlan *P)
     P->fix = tg_plan_fix(S);
     // (the dense linear algebra strides over the free variables: a warp once they are more than 32)
     P->lanes = L.n > 32 ? 32 : tg_default_gs(L);
-    P->per_bytes = tg_polish_group_doubles(L) * sizeof(double);
+    P->per_bytes = per_doubles * sizeof(double);
     const size_t fit = ((size_t)g_smem_optin - 1024) / P->per_bytes;
     const char *v = getenv("TG_POLISH_FAR");
     P->far = fit == 0 || (v && atoi(v) != 0);
@@ -974,11 +975,19 @@ static int tg_plan_polish(const TgShape &S, int B, TgPolishPlan *P)
     return 0;
 }
 
+// the five fields of tg_polish_plan_info / tg_sens_plan_info
+static int tg_plan_info_out(const TgPolishPlan &P, int *out, int cap)
+{
+    const int v[5] = {P.lanes, P.far, P.groups, P.grid, (int)(P.per_bytes >> 10)};
+    for (int i = 0; i < 5 && out && i < cap; i++) out[i] = v[i];
+    return 5;
+}
+
 extern "C" size_t tg_polish_workspace_bytes(const int *spec, int B)
 {
     TgShape S;
     TgPolishPlan P;
-    if (tg_make_shape(spec, &S) || tg_plan_polish(S, B > 0 ? B : 1, &P)) return 0;
+    if (tg_make_shape(spec, &S) || tg_plan_polish(S, B > 0 ? B : 1, tg_polish_group_doubles(S.L), &P)) return 0;
     return P.ws_bytes;
 }
 
@@ -987,11 +996,9 @@ extern "C" int tg_polish_plan_info(const int *spec, int B, int *out, int cap)
     TgShape S;
     TgPolishPlan P;
     int rc = tg_make_shape(spec, &S);
-    if (!rc) rc = tg_plan_polish(S, B > 0 ? B : 1, &P);
+    if (!rc) rc = tg_plan_polish(S, B > 0 ? B : 1, tg_polish_group_doubles(S.L), &P);
     if (rc) return -rc;
-    const int v[5] = {P.lanes, P.far, P.groups, P.grid, (int)(P.per_bytes >> 10)};
-    for (int i = 0; i < 5 && out && i < cap; i++) out[i] = v[i];
-    return 5;
+    return tg_plan_info_out(P, out, cap);
 }
 
 extern "C" int tg_polish_batch(const int *spec, int B, const double *par, double *x, double *f, const int *status,
@@ -1005,7 +1012,7 @@ extern "C" int tg_polish_batch(const int *spec, int B, const double *par, double
     if (!par || !x || !f || !status || !violation || !lam || !kkt || !polish_status || !polish_iters)
         return tg_fail(1, "tg_polish_batch: NULL argument");
     TgPolishPlan P;
-    if ((rc = tg_plan_polish(S, B, &P))) return rc;
+    if ((rc = tg_plan_polish(S, B, tg_polish_group_doubles(S.L), &P))) return rc;
     if (P.ws_bytes && (!ws || ws_bytes < P.ws_bytes)) return tg_fail(4, "workspace too small (see tg_polish_workspace_bytes)");
     const TgPolishLaunch a = {S, B, par, x, f, status, violation, lam, kkt, polish_status, polish_iters, maxiter, tol,
                               P.far ? (double *)ws : nullptr, P.fix, P.grid, P.groups, P.smem, (cudaStream_t)stream};
@@ -1013,6 +1020,46 @@ extern "C" int tg_polish_batch(const int *spec, int B, const double *par, double
     cudaError_t e = launchers[tg_lanes_index(P.lanes)](a);
     g_launches++;
     if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_polish_kernel launch", e);
+    return 0;
+}
+
+extern "C" size_t tg_sens_workspace_bytes(const int *spec, int B)
+{
+    TgShape S;
+    TgPolishPlan P;
+    if (tg_make_shape(spec, &S) || tg_plan_polish(S, B > 0 ? B : 1, tg_sens_group_doubles(S.L), &P)) return 0;
+    return P.ws_bytes;
+}
+
+extern "C" int tg_sens_plan_info(const int *spec, int B, int *out, int cap)
+{
+    TgShape S;
+    TgPolishPlan P;
+    int rc = tg_make_shape(spec, &S);
+    if (!rc) rc = tg_plan_polish(S, B > 0 ? B : 1, tg_sens_group_doubles(S.L), &P);
+    if (rc) return -rc;
+    return tg_plan_info_out(P, out, cap);
+}
+
+extern "C" int tg_sens_batch(const int *spec, int B, const double *par, const double *x, const int *status,
+                             const double *lam, const double *x_bar, const double *f_bar, double *par_bar,
+                             int *sens_status, double tol, void *ws, size_t ws_bytes, void *stream)
+{
+    TgShape S;
+    int rc = tg_make_shape(spec, &S);
+    if (rc) return rc;
+    if (B <= 0) return 0;
+    if (!par || !x || !status || !lam || !x_bar || !par_bar || !sens_status)
+        return tg_fail(1, "tg_sens_batch: NULL argument");
+    TgPolishPlan P;
+    if ((rc = tg_plan_polish(S, B, tg_sens_group_doubles(S.L), &P))) return rc;
+    if (P.ws_bytes && (!ws || ws_bytes < P.ws_bytes)) return tg_fail(4, "workspace too small (see tg_sens_workspace_bytes)");
+    const TgSensLaunch a = {S, B, par, x, status, lam, x_bar, f_bar, par_bar, sens_status, tol,
+                            P.far ? (double *)ws : nullptr, P.fix, P.grid, P.groups, P.smem, (cudaStream_t)stream};
+    static cudaError_t (*const launchers[3])(const TgSensLaunch &) = {tg_launch_sens_g8, tg_launch_sens_g16, tg_launch_sens_g32};
+    cudaError_t e = launchers[tg_lanes_index(P.lanes)](a);
+    g_launches++;
+    if (e != cudaSuccess) return tg_fail(100 + (int)e, "tg_sens_kernel launch", e);
     return 0;
 }
 

@@ -1,5 +1,6 @@
 // Post-solve polish of a converged problem: safeguarded Newton steps on the KKT system of SLSQP's final active set with
 // an exact Lagrangian Hessian (tg_polish_kernel, tg_kernels_polish.inc; the host build under tests/hostsim).
+// The parameter sensitivities (tg_sens.h) call its working set, Hessian, QR and Cholesky functions as well.
 //
 // SLSQP stops when |f - f0| or the step falls below its tolerance.  A badly conditioned BFGS factor makes the step tiny
 // while the Lagrangian gradient is still large, so a status-0 point is feasible and complementary but often not
@@ -170,6 +171,204 @@ TG_HD void tg_polish_reflect(const TgPolishWs &P, int nF, int k, double *vec)
     for (int a = k; a < nF; a++) vec[a] -= s * v[a];
 }
 
+// free variables (P.fr, x strictly inside its bounds) and working set (P.wrow: every equality row and the inequality
+// rows with lam_j > 0 not marked in P.drop), both in index order; every lane
+TG_HD void tg_polish_sets(const TgLayout &L, const TgPolishWs &P, int *nFo, int *nWo)
+{
+    const int lane = TG_LANE();
+    int nF = 0, nW = 0;
+    #pragma unroll 1
+    for (int i = 0; i < L.n; i++)
+        if (P.x[i] != P.xl[i] && P.x[i] != P.xu[i]) { if (lane == 0) P.fr[nF] = i; nF++; }
+    #pragma unroll 1
+    for (int j = 0; j < L.m; j++)
+        if (j < L.meq || (P.lam[j] > 0 && !P.drop[j])) { if (lane == 0) P.wrow[nW] = j; nW++; }
+    TG_SYNC();
+    *nFo = nF; *nWo = nW;
+}
+
+// H (nF x nF, row-major) = d2L/dx2 over the free variables at P.x with the multipliers P.lam: column b from
+// tg_polish_gradl at x +- h e_i, h = eps^(1/3) max(1, |x_i|), one-sided at a bound; symmetrised
+template <int D>
+TG_FN void tg_polish_hessian(const TgLayout &L, const int *sp, const TgPolishWs &P, int nF)
+{
+    const int lane = TG_LANE();
+    #pragma unroll 1
+    for (int b = 0; b < nF; b++) {
+        const int i = P.fr[b];
+        const double xi = P.x[i], h = TG_POLISH_H_REL * fmax(1.0, fabs(xi));
+        const double xp = fmin(xi + h, P.xu[i]), xm = fmax(xi - h, P.xl[i]);
+        if (lane == 0) P.xt[i] = xp;
+        TG_SYNC();
+        tg_polish_gradl<D>(L, sp, P, nF);
+        #pragma unroll 1
+        for (int a = lane; a < nF; a += TG_NL) P.H[(size_t)a * nF + b] = P.gp[a];
+        if (lane == 0) P.xt[i] = xm;
+        TG_SYNC();
+        tg_polish_gradl<D>(L, sp, P, nF);
+        #pragma unroll 1
+        for (int a = lane; a < nF; a += TG_NL) P.H[(size_t)a * nF + b] = (P.H[(size_t)a * nF + b] - P.gp[a]) / (xp - xm);
+        if (lane == 0) P.xt[i] = xi;
+        TG_SYNC();
+    }
+    #pragma unroll 1
+    for (int a = lane; a < nF; a += TG_NL)
+        #pragma unroll 1
+        for (int b = a + 1; b < nF; b++) {
+            const double s = 0.5 * (P.H[(size_t)a * nF + b] + P.H[(size_t)b * nF + a]);
+            P.H[(size_t)a * nF + b] = s; P.H[(size_t)b * nF + a] = s;
+        }
+    TG_SYNC();
+}
+
+// Householder QR of A_W' (nF x nW, column k = Jacobian row W_k over the free variables) in place in P.AT: reflector k
+// is AT column k from entry k on with P.beta[k]; R_kk = rdiag[k], R_kj = AT[j][k] (j > k).  Returns 1 when A_W is
+// rank-deficient (some |R_kk| < 1e-12 max|R|); every lane
+TG_FN int tg_polish_qr(const TgLayout &L, const TgPolishWs &P, int nF, int nW)
+{
+    const int lane = TG_LANE(), n = L.n;
+    #pragma unroll 1
+    for (int q = lane; q < nF * nW; q += TG_NL) {
+        const int k = q / nF, a = q - k * nF;
+        P.AT[q] = P.J[(size_t)P.wrow[k] * n + P.fr[a]];
+    }
+    TG_SYNC();
+    #pragma unroll 1
+    for (int k = 0; k < nW; k++) {
+        double *v = P.AT + (size_t)k * nF;
+        double s = 0;
+        #pragma unroll 1
+        for (int a = k; a < nF; a++) s += v[a] * v[a];
+        const double nrm = sqrt(s), vk0 = v[k];
+        const double alpha = vk0 > 0 ? -nrm : nrm, vk = vk0 - alpha;
+        const double beta = nrm > 0 ? -1.0 / (alpha * vk) : 0.0;
+        TG_SYNC();
+        if (lane == 0) { v[k] = vk; P.beta[k] = beta; P.rdiag[k] = alpha; }
+        TG_SYNC();
+        #pragma unroll 1
+        for (int j = k + 1 + lane; j < nW; j += TG_NL) {
+            double *col = P.AT + (size_t)j * nF;
+            double t = 0;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) t += v[a] * col[a];
+            t *= beta;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) col[a] -= t * v[a];
+        }
+        TG_SYNC();
+    }
+    double rmax = 0;
+    #pragma unroll 1
+    for (int q = lane; q < nW * nW; q += TG_NL) {
+        const int j = q / nW, k = q - j * nW;
+        if (k < j) rmax = tg_kkt_fold(rmax, fabs(P.AT[(size_t)j * nF + k]));
+        else if (k == j) rmax = tg_kkt_fold(rmax, fabs(P.rdiag[k]));
+    }
+    int k0 = 0;
+    tg_wargmax(rmax, k0);
+    int rankdef = 0;
+    #pragma unroll 1
+    for (int k = 0; k < nW; k++) rankdef |= !(fabs(P.rdiag[k]) >= 1e-12 * rmax);
+    return rankdef;
+}
+
+// C = Q'HQ (reflector k from the left on every column, then from the right on every row); returns max|H|; every lane
+TG_FN double tg_polish_reduce(const TgPolishWs &P, int nF, int nW)
+{
+    const int lane = TG_LANE();
+    double hmax = 0;
+    #pragma unroll 1
+    for (size_t q = lane; q < (size_t)nF * nF; q += TG_NL) { P.C[q] = P.H[q]; hmax = tg_kkt_fold(hmax, fabs(P.H[q])); }
+    int k0 = 0;
+    tg_wargmax(hmax, k0);
+    TG_SYNC();
+    #pragma unroll 1
+    for (int k = 0; k < nW; k++) {
+        const double *v = P.AT + (size_t)k * nF, beta = P.beta[k];
+        #pragma unroll 1
+        for (int j = lane; j < nF; j += TG_NL) {
+            double t = 0;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) t += v[a] * P.C[(size_t)a * nF + j];
+            t *= beta;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) P.C[(size_t)a * nF + j] -= t * v[a];
+        }
+        TG_SYNC();
+        #pragma unroll 1
+        for (int i = lane; i < nF; i += TG_NL) {
+            double *row = P.C + (size_t)i * nF;
+            double t = 0;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) t += row[a] * v[a];
+            t *= beta;
+            #pragma unroll 1
+            for (int a = k; a < nF; a++) row[a] -= t * v[a];
+        }
+        TG_SYNC();
+    }
+    return hmax;
+}
+
+// Cholesky of the reduced Hessian C[nW.., nW..] + delta I into F (lower triangle, row-major nz x nz, nz = nF - nW);
+// returns 0 when a pivot is not positive and finite; every lane
+TG_FN int tg_polish_chol(const TgPolishWs &P, int nF, int nW, double delta)
+{
+    const int lane = TG_LANE(), nz = nF - nW;
+    #pragma unroll 1
+    for (int q = lane; q < nz * nz; q += TG_NL) {
+        const int a = q / nz, b = q - a * nz;
+        P.F[q] = P.C[(size_t)(nW + a) * nF + nW + b] + (a == b ? delta : 0.0);
+    }
+    TG_SYNC();
+    int ok = 1;
+    #pragma unroll 1
+    for (int k = 0; k < nz && ok; k++) {
+        const double d = P.F[(size_t)k * nz + k];
+        if (!(d > 0) || !tg_finite(d)) { ok = 0; break; }
+        const double lkk = sqrt(d);
+        TG_SYNC();
+        if (lane == 0) P.F[(size_t)k * nz + k] = lkk;
+        #pragma unroll 1
+        for (int i = k + 1 + lane; i < nz; i += TG_NL) P.F[(size_t)i * nz + k] /= lkk;
+        TG_SYNC();
+        #pragma unroll 1
+        for (int i = k + 1 + lane; i < nz; i += TG_NL) {
+            const double lik = P.F[(size_t)i * nz + k];
+            #pragma unroll 1
+            for (int j = k + 1; j <= i; j++) P.F[(size_t)i * nz + j] -= lik * P.F[(size_t)j * nz + k];
+        }
+        TG_SYNC();
+    }
+    TG_SYNC();
+    return ok;
+}
+
+// vec[0..nz) <- (F F')^-1 vec, forward then back substitution; one lane
+TG_HD void tg_polish_chol_solve(const TgPolishWs &P, int nz, double *vec)
+{
+    for (int a = 0; a < nz; a++) {
+        double s = vec[a];
+        for (int b = 0; b < a; b++) s -= P.F[(size_t)a * nz + b] * vec[b];
+        vec[a] = s / P.F[(size_t)a * nz + a];
+    }
+    for (int a = nz - 1; a >= 0; a--) {
+        double s = vec[a];
+        for (int b = a + 1; b < nz; b++) s -= P.F[(size_t)b * nz + a] * vec[b];
+        vec[a] = s / P.F[(size_t)a * nz + a];
+    }
+}
+
+// vec[0..nW) <- R^-1 vec, back substitution with the R of tg_polish_qr; one lane
+TG_HD void tg_polish_rsolve(const TgPolishWs &P, int nF, int nW, double *vec)
+{
+    for (int k = nW - 1; k >= 0; k--) {
+        double s = vec[k];
+        for (int j = k + 1; j < nW; j++) s -= P.AT[(size_t)j * nF + k] * vec[j];
+        vec[k] = s / P.rdiag[k];
+    }
+}
+
 // Polishes one problem in place (see the top of the file).  sp / par: the problem's descriptor and parameter row;
 // x[n], f, violation, lam[m], kkt[4]: its solve outputs, replaced only when the final guard holds.
 template <int D>
@@ -214,126 +413,24 @@ TG_FN void tg_polish_problem(const TgLayout &L, const int *sp, const double *par
         if (kkt[0] <= tol * fmax(1.0, gmax)) { conv = 1; break; }
         if (it >= maxiter) break;
         // ---- free variables and working set
-        int nF = 0, nW = 0;
-        #pragma unroll 1
-        for (int i = 0; i < n; i++)
-            if (P.x[i] != P.xl[i] && P.x[i] != P.xu[i]) { if (lane == 0) P.fr[nF] = i; nF++; }
-        #pragma unroll 1
-        for (int j = 0; j < m; j++)
-            if (j < meq || (P.lam[j] > 0 && !P.drop[j])) { if (lane == 0) P.wrow[nW] = j; nW++; }
-        TG_SYNC();
+        int nF, nW;
+        tg_polish_sets(L, P, &nF, &nW);
         if (nW > nF) {
             if (lane == 0) { *pstatus = TG_POLISH_DEGENERATE; *piters = it; }
             return;
         }
-        // ---- Hessian of the Lagrangian over the free variables: column b from gradL at x +- h e_i
+        // ---- Hessian of the Lagrangian over the free variables
         if (!hvalid) {
-            #pragma unroll 1
-            for (int b = 0; b < nF; b++) {
-                const int i = P.fr[b];
-                const double xi = P.x[i], h = TG_POLISH_H_REL * fmax(1.0, fabs(xi));
-                const double xp = fmin(xi + h, P.xu[i]), xm = fmax(xi - h, P.xl[i]);
-                if (lane == 0) P.xt[i] = xp;
-                TG_SYNC();
-                tg_polish_gradl<D>(L, sp, P, nF);
-                #pragma unroll 1
-                for (int a = lane; a < nF; a += TG_NL) P.H[(size_t)a * nF + b] = P.gp[a];
-                if (lane == 0) P.xt[i] = xm;
-                TG_SYNC();
-                tg_polish_gradl<D>(L, sp, P, nF);
-                #pragma unroll 1
-                for (int a = lane; a < nF; a += TG_NL) P.H[(size_t)a * nF + b] = (P.H[(size_t)a * nF + b] - P.gp[a]) / (xp - xm);
-                if (lane == 0) P.xt[i] = xi;
-                TG_SYNC();
-            }
-            #pragma unroll 1
-            for (int a = lane; a < nF; a += TG_NL)
-                #pragma unroll 1
-                for (int b = a + 1; b < nF; b++) {
-                    const double s = 0.5 * (P.H[(size_t)a * nF + b] + P.H[(size_t)b * nF + a]);
-                    P.H[(size_t)a * nF + b] = s; P.H[(size_t)b * nF + a] = s;
-                }
-            TG_SYNC();
+            tg_polish_hessian<D>(L, sp, P, nF);
             hvalid = 1;
         }
-        // (the null-space step transforms a copy: C holds Q'HQ)
-        double hmax = 0;
-        #pragma unroll 1
-        for (size_t q = lane; q < (size_t)nF * nF; q += TG_NL) { P.C[q] = P.H[q]; hmax = tg_kkt_fold(hmax, fabs(P.H[q])); }
-        tg_wargmax(hmax, k0);
         // ---- Householder QR of A_W' (nF x nW, column k = row W_k over the free variables)
-        #pragma unroll 1
-        for (int q = lane; q < nF * nW; q += TG_NL) {
-            const int k = q / nF, a = q - k * nF;
-            P.AT[q] = P.J[(size_t)P.wrow[k] * n + P.fr[a]];
-        }
-        TG_SYNC();
-        #pragma unroll 1
-        for (int k = 0; k < nW; k++) {
-            double *v = P.AT + (size_t)k * nF;
-            double s = 0;
-            #pragma unroll 1
-            for (int a = k; a < nF; a++) s += v[a] * v[a];
-            const double nrm = sqrt(s), vk0 = v[k];
-            const double alpha = vk0 > 0 ? -nrm : nrm, vk = vk0 - alpha;
-            const double beta = nrm > 0 ? -1.0 / (alpha * vk) : 0.0;
-            TG_SYNC();
-            if (lane == 0) { v[k] = vk; P.beta[k] = beta; P.rdiag[k] = alpha; }
-            TG_SYNC();
-            #pragma unroll 1
-            for (int j = k + 1 + lane; j < nW; j += TG_NL) {
-                double *col = P.AT + (size_t)j * nF;
-                double t = 0;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) t += v[a] * col[a];
-                t *= beta;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) col[a] -= t * v[a];
-            }
-            TG_SYNC();
-        }
-        // rank: R_kk = rdiag[k], R_kj = AT[j][k] (j > k)
-        double rmax = 0;
-        #pragma unroll 1
-        for (int q = lane; q < nW * nW; q += TG_NL) {
-            const int j = q / nW, k = q - j * nW;
-            if (k < j) rmax = tg_kkt_fold(rmax, fabs(P.AT[(size_t)j * nF + k]));
-            else if (k == j) rmax = tg_kkt_fold(rmax, fabs(P.rdiag[k]));
-        }
-        tg_wargmax(rmax, k0);
-        int rankdef = 0;
-        #pragma unroll 1
-        for (int k = 0; k < nW; k++) rankdef |= !(fabs(P.rdiag[k]) >= 1e-12 * rmax);
-        if (rankdef) {
+        if (tg_polish_qr(L, P, nF, nW)) {
             if (lane == 0) { *pstatus = TG_POLISH_DEGENERATE; *piters = it; }
             return;
         }
-        // ---- C = Q'HQ (reflector k from the left on every column, then from the right on every row), gq = Q'g_F
-        #pragma unroll 1
-        for (int k = 0; k < nW; k++) {
-            const double *v = P.AT + (size_t)k * nF, beta = P.beta[k];
-            #pragma unroll 1
-            for (int j = lane; j < nF; j += TG_NL) {
-                double t = 0;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) t += v[a] * P.C[(size_t)a * nF + j];
-                t *= beta;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) P.C[(size_t)a * nF + j] -= t * v[a];
-            }
-            TG_SYNC();
-            #pragma unroll 1
-            for (int i = lane; i < nF; i += TG_NL) {
-                double *row = P.C + (size_t)i * nF;
-                double t = 0;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) t += row[a] * v[a];
-                t *= beta;
-                #pragma unroll 1
-                for (int a = k; a < nF; a++) row[a] -= t * v[a];
-            }
-            TG_SYNC();
-        }
+        // ---- C = Q'HQ, gq = Q'g_F
+        const double hmax = tg_polish_reduce(P, nF, nW);
         if (lane == 0) {
             for (int a = 0; a < nF; a++) P.gq[a] = P.g[P.fr[a]];
             for (int k = 0; k < nW; k++) tg_polish_reflect(P, nF, k, P.gq);
@@ -345,39 +442,12 @@ TG_FN void tg_polish_problem(const TgLayout &L, const int *sp, const double *par
             }
         }
         TG_SYNC();
-        // ---- reduced Hessian C[nW.., nW..] + delta I, Cholesky into F (lower triangle, row-major nz x nz)
+        // ---- reduced Hessian C[nW.., nW..] + delta I, Cholesky into F
         const int nz = nF - nW;
         int chol_ok = nz == 0;
         #pragma unroll 1
-        for (int attempt = 0; attempt < 4 && !chol_ok; attempt++) {
-            const double delta = attempt == 0 ? 0.0 : 1e-8 * hmax * (attempt == 1 ? 1.0 : attempt == 2 ? 1e2 : 1e4);
-            #pragma unroll 1
-            for (int q = lane; q < nz * nz; q += TG_NL) {
-                const int a = q / nz, b = q - a * nz;
-                P.F[q] = P.C[(size_t)(nW + a) * nF + nW + b] + (a == b ? delta : 0.0);
-            }
-            TG_SYNC();
-            chol_ok = 1;
-            #pragma unroll 1
-            for (int k = 0; k < nz && chol_ok; k++) {
-                const double d = P.F[(size_t)k * nz + k];
-                if (!(d > 0) || !tg_finite(d)) { chol_ok = 0; break; }
-                const double lkk = sqrt(d);
-                TG_SYNC();
-                if (lane == 0) P.F[(size_t)k * nz + k] = lkk;
-                #pragma unroll 1
-                for (int i = k + 1 + lane; i < nz; i += TG_NL) P.F[(size_t)i * nz + k] /= lkk;
-                TG_SYNC();
-                #pragma unroll 1
-                for (int i = k + 1 + lane; i < nz; i += TG_NL) {
-                    const double lik = P.F[(size_t)i * nz + k];
-                    #pragma unroll 1
-                    for (int j = k + 1; j <= i; j++) P.F[(size_t)i * nz + j] -= lik * P.F[(size_t)j * nz + k];
-                }
-                TG_SYNC();
-            }
-            TG_SYNC();
-        }
+        for (int attempt = 0; attempt < 4 && !chol_ok; attempt++)
+            chol_ok = tg_polish_chol(P, nF, nW, attempt == 0 ? 0.0 : 1e-8 * hmax * (attempt == 1 ? 1.0 : attempt == 2 ? 1e2 : 1e4));
         if (!chol_ok) break;
         // null-space part: (Z'HZ) p_z = -(gq_z + C_zy p_y); rhs in tmp
         #pragma unroll 1
@@ -390,16 +460,7 @@ TG_FN void tg_polish_problem(const TgLayout &L, const int *sp, const double *par
         }
         TG_SYNC();
         if (lane == 0) {
-            for (int a = 0; a < nz; a++) {
-                double s = P.tmp[a];
-                for (int b = 0; b < a; b++) s -= P.F[(size_t)a * nz + b] * P.tmp[b];
-                P.tmp[a] = s / P.F[(size_t)a * nz + a];
-            }
-            for (int a = nz - 1; a >= 0; a--) {
-                double s = P.tmp[a];
-                for (int b = a + 1; b < nz; b++) s -= P.F[(size_t)b * nz + a] * P.tmp[b];
-                P.tmp[a] = s / P.F[(size_t)a * nz + a];
-            }
+            tg_polish_chol_solve(P, nz, P.tmp);
             for (int a = 0; a < nz; a++) P.pq[nW + a] = P.tmp[a];
         }
         TG_SYNC();
@@ -414,11 +475,7 @@ TG_FN void tg_polish_problem(const TgLayout &L, const int *sp, const double *par
         }
         TG_SYNC();
         if (lane == 0) {
-            for (int k = nW - 1; k >= 0; k--) {
-                double s = P.tmp[k];
-                for (int j = k + 1; j < nW; j++) s -= P.AT[(size_t)j * nF + k] * P.tmp[j];
-                P.tmp[k] = s / P.rdiag[k];
-            }
+            tg_polish_rsolve(P, nF, nW, P.tmp);
             for (int j = 0; j < m; j++) P.lamw[j] = 0;
             for (int k = 0; k < nW; k++) P.lamw[P.wrow[k]] = P.tmp[k];
             // step over the free variables: p_F = Q pq

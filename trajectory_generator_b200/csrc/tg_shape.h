@@ -190,6 +190,24 @@ struct TgPolishLaunch {
 };
 cudaError_t tg_launch_polish_g8(const TgPolishLaunch &a), tg_launch_polish_g16(const TgPolishLaunch &a),
     tg_launch_polish_g32(const TgPolishLaunch &a);
+// Parameter-sensitivity kernel (tg_kernels_sens.inc, planned by tg_plan_polish with tg_sens_group_doubles of scratch);
+// f_bar may be nullptr (zeros)
+struct TgSensLaunch {
+    TgShape S;
+    int B;
+    const double *par, *x;
+    const int *status;
+    const double *lam, *x_bar, *f_bar;
+    double *par_bar;
+    int *sens_status;
+    double tol;
+    double *far;
+    int fix, grid, groups;
+    size_t smem;
+    cudaStream_t st;
+};
+cudaError_t tg_launch_sens_g8(const TgSensLaunch &a), tg_launch_sens_g16(const TgSensLaunch &a),
+    tg_launch_sens_g32(const TgSensLaunch &a);
 // Multi-start expansion (tg_multistart.cu)
 cudaError_t tg_launch_multistart_expand(const TgLayout &L, int B, int K, const double *par, const double *x0,
                                         unsigned long long seed, double spread, double *par_out, double *x_out,
